@@ -32,6 +32,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # a run leaves the tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -158,6 +159,25 @@ def toxic(seed):
     return [rng.next_fr() for _ in range(5)]
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, proofs, status):
+    """--dump-outputs: the proofs (n x 256 bytes) and status codes a caller of the timed path receives, as float32
+    path/proofs.npy and path/status.npy (exact: bytes and small integers), plus path/rows.npy (float64), the batch rows
+    written: all of them while the files fit in 64 MiB, else a fixed seeded sample.  Inputs are seeded, so two builds
+    run with the same arguments can be compared file for file."""
+    n = len(proofs)
+    row_bytes = 4 * proofs.shape[1] + 4 + 8
+    rows = np.arange(n)
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "proofs.npy"), proofs[rows].astype(np.float32))
+    np.save(os.path.join(path, "status.npy"), status[rows].astype(np.float32))
+    np.save(os.path.join(path, "rows.npy"), rows.astype(np.float64))
+
+
 # ----------------------------------------------------------------------------- reference arm (CPU)
 def host_cores():
     """Host threads this process may use.  torchrun exports OMP_NUM_THREADS=1 to every rank, which made the OpenMP
@@ -191,6 +211,8 @@ def run_reference(args, rank, world):
         proofs, status = co.prove_batch(circ, opk, a, a, None, None, r, s, threads=cores)
     dt = time.perf_counter() - t0
     assert not status.any()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proofs, status)
     v = sample * args.steps / dt
     desc = (f"each step proves the first {sample} of the batch's {args.batch} independent equality proofs, "
             f"proof-parallel over {cores} OpenMP threads (explicit; OMP_NUM_THREADS is ignored)")
@@ -288,6 +310,8 @@ def run_ours(args, rank, world, local_rank):
     ms = ev0.elapsed_time(ev1)
     launches = engine.kernel_launches() - launches0
     clocks = sampler.stop(w0, w1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_proofs.cpu().numpy(), d_status.cpu().numpy())
     regions = pk.profile_read(reset=True)
     engine.profile_enable(False)
     if world > 1:
@@ -694,6 +718,8 @@ def main():
     ap.add_argument("--ref-sample", type=int, default=0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's proofs and "
+                    "status codes (rank 0's) as .npy files in DIR")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
