@@ -103,11 +103,11 @@ struct MsmPlan {                 // one curve
     DBuf items[4];               // uint2[n_items[v]] for the four granularities
     DBuf msm_items[4];           // uint2[n_msm]: item range of each MSM
     uint32_t n_items[4] = {0, 0, 0, 0};
+    uint32_t item_len[4] = {8, 32, 128, 512};   // units per item of each granularity
     uint32_t n_units = 0, n_rows = 0, n_msm = 0;
     std::vector<uint32_t> msm_unit_begin;   // host: first unit of each MSM (+ end)
     std::vector<uint2> msm_items_host[4];   // host copy of msm_items per granularity
 };
-static const uint32_t kUnitsPerItem[4] = {8, 32, 128, 512};
 
 // Host memory the device can DMA to without an intermediate copy (results of a chunk land here asynchronously).
 struct HBuf {
@@ -241,8 +241,8 @@ static int finish_plan(MsmPlan &pl, const std::vector<std::vector<BaseRef>> &msm
         std::vector<uint2> items, mi;
         for (uint32_t q = 0; q < pl.n_msm; q++) {
             uint32_t first = (uint32_t)items.size();
-            for (uint32_t u = pl.msm_unit_begin[q]; u < pl.msm_unit_begin[q + 1]; u += kUnitsPerItem[v])
-                items.push_back(make_uint2(u, std::min(u + kUnitsPerItem[v], pl.msm_unit_begin[q + 1])));
+            for (uint32_t u = pl.msm_unit_begin[q]; u < pl.msm_unit_begin[q + 1]; u += pl.item_len[v])
+                items.push_back(make_uint2(u, std::min(u + pl.item_len[v], pl.msm_unit_begin[q + 1])));
             mi.push_back(make_uint2(first, (uint32_t)items.size()));
         }
         pl.n_items[v] = (uint32_t)items.size();
@@ -251,6 +251,23 @@ static int finish_plan(MsmPlan &pl, const std::vector<std::vector<BaseRef>> &msm
         TRY(upload(pl.msm_items[v], mi));
     }
     return LZKP_OK;
+}
+
+// Units per item of the large-batch G1 grid (granularity 2: dim3(P / 128, items) of 128-thread CTAs of nearly equal
+// length).  Such a grid runs in whole waves of the resident CTAs, so a last wave that is barely filled costs as much
+// as a full one: the length is the one in [96, 192] with the least (waves rounded up) x (units per item), summed over
+// batches of 1024 to 8192 proofs.  (The equality key at c = 17 with 128-unit items: 5312 CTAs = 8.97 waves of 592;
+// after the shared A/B1 terms 4928 = 8.32 waves, still paying for 9; at 133 units 4736 = 8.00 waves.)
+static uint32_t fit_item_len(const std::vector<std::vector<BaseRef>> &msms, uint32_t W, uint32_t resident) {
+    uint32_t best = 128;
+    uint64_t best_cost = UINT64_MAX;
+    for (uint32_t len = 96; len <= 192; len++) {
+        uint64_t items = 0, cost = 0;
+        for (auto &ms : msms) items += ((uint64_t)ms.size() * W + len - 1) / len;
+        for (uint64_t gx : {8u, 16u, 32u, 64u}) cost += (gx * items + resident - 1) / resident * len * (64 / gx);
+        if (cost < best_cost) { best_cost = cost; best = len; }
+    }
+    return best;
 }
 
 // Signed c-bit windows of an Fr scalar by the offset trick (dev_util.cuh recode_offset): s + K must stay below
@@ -491,12 +508,27 @@ static int pk_load_impl(const uint8_t *bytes, size_t len, int validate, const lz
     }
 
     // --- base lists (identity points are dropped: they contribute nothing to any MSM) ---
+    // A variable whose A and B1 query points are the same point adds the same term z_j a_j to the A sum and to the
+    // B1 sum (every MiMC-5 round of libzkp's circuits: A column = B column for t2 = t*t): the batch form computes it
+    // once, in MSM 4 ("shared", one table row), and k_assemble adds that sum to both.
     std::vector<host::G1Canon> rows1;
     std::vector<host::G2Canon> rows2;
-    std::vector<std::vector<BaseRef>> msm1(4), msm2(1);
+    std::vector<std::vector<BaseRef>> msm1(5), msm2(1);
+    std::vector<BaseRef> a_all, b1_all;              // every a / b1 term, shared ones included (latency form)
     auto add1 = [&](const host::G1Canon &p) { rows1.push_back(p); return (uint32_t)rows1.size() - 1; };
-    for (uint32_t j = 1; j < nv; j++) if (!host::is_inf(a_q[j])) msm1[0].push_back({j - 1, add1(a_q[j])});
-    for (uint32_t j = 1; j < nv; j++) if (!host::is_inf(b1_q[j])) msm1[1].push_back({j - 1, add1(b1_q[j])});
+    auto same_point = [](const host::G1Canon &u, const host::G1Canon &v) {
+        return memcmp(&u.x, &v.x, sizeof(Fq)) == 0 && memcmp(&u.y, &v.y, sizeof(Fq)) == 0;
+    };
+    for (uint32_t j = 1; j < nv; j++) {
+        const bool has_a = !host::is_inf(a_q[j]), has_b = !host::is_inf(b1_q[j]);
+        if (has_a && has_b && same_point(a_q[j], b1_q[j])) {
+            const BaseRef ref{j - 1, add1(a_q[j])};
+            msm1[4].push_back(ref); a_all.push_back(ref); b1_all.push_back(ref);
+            continue;
+        }
+        if (has_a) { msm1[0].push_back({j - 1, add1(a_q[j])}); a_all.push_back(msm1[0].back()); }
+        if (has_b) { msm1[1].push_back({j - 1, add1(b1_q[j])}); b1_all.push_back(msm1[1].back()); }
+    }
     for (uint32_t j = 0; j < pk->n_wit; j++) if (!host::is_inf(l_q[j])) msm1[2].push_back({pk->n_inst + j - 1, add1(l_q[j])});
     for (uint32_t i = 0; i + 1 < n; i++) if (!host::is_inf(h_q[i])) msm1[3].push_back({ROW_H + i, add1(h_q[i])});
     if (!host::is_inf(delta_g1)) {
@@ -504,16 +536,19 @@ static int pk_load_impl(const uint8_t *bytes, size_t len, int validate, const lz
         msm1[0].push_back({ROW_R, rd1});      // A  += r * delta_g1
         msm1[1].push_back({ROW_S, rd1});      // B1 += s * delta_g1
         msm1[2].push_back({ROW_RS, rnd1});    // C  -= rs * delta_g1 (folded into the L sum)
+        a_all.push_back({ROW_R, rd1});
     }
-    // latency form: C = s*(alpha + a0) + r*(beta + b0) + sum (s z_i) a_i + sum (r z_i) b_i + 2 rs delta + [L - rs delta] + H
-    std::vector<std::vector<BaseRef>> msm1_lat;
+    // latency form: C = s*(alpha + a0) + r*(beta + b0) + sum (s z_i) a_i + sum (r z_i) b_i + 2 rs delta + [L - rs delta] + H.
+    // The proof needs the A sum itself (slot 0, whole: no shared MSM) but B1 only as r*B1 (slot 5), so slot 1 stays empty.
+    std::vector<std::vector<BaseRef>> msm1_lat(6);
     {
         pk->row_sz = pk->n_dig_rows;
         pk->row_rz = pk->n_dig_rows + pk->nz;
-        msm1_lat = msm1;
-        msm1_lat.resize(6);
-        for (auto &b : msm1[0]) if (b.dig_row < pk->nz) msm1_lat[4].push_back({pk->row_sz + b.dig_row, b.tbl_row});
-        for (auto &b : msm1[1]) if (b.dig_row < pk->nz) msm1_lat[5].push_back({pk->row_rz + b.dig_row, b.tbl_row});
+        msm1_lat[0] = a_all;
+        msm1_lat[2] = msm1[2];
+        msm1_lat[3] = msm1[3];
+        for (auto &b : a_all) if (b.dig_row < pk->nz) msm1_lat[4].push_back({pk->row_sz + b.dig_row, b.tbl_row});
+        for (auto &b : b1_all) msm1_lat[5].push_back({pk->row_rz + b.dig_row, b.tbl_row});
         // the three constant points, computed with the host build of the same field / curve code
         auto mont = [](const host::G1Canon &c) { return G1Affine{Fq::from_canonical(c.x), Fq::from_canonical(c.y)}; };
         auto canon = [](const G1Affine &m) { host::G1Canon c; c.x = m.x.to_canonical(); c.y = m.y.to_canonical(); return c; };
@@ -619,6 +654,11 @@ static int pk_load_impl(const uint8_t *bytes, size_t len, int validate, const lz
         TRY(build_table_g1(d_rows1.p, (uint32_t)rows1.size(), c, pk->W, pk->N, pk->g1.table.p, st));
     if (!rows2.empty())
         TRY(build_table_g2(d_rows2.p, (uint32_t)rows2.size(), c, pk->W, pk->N, pk->g2.table.p, st));
+    {
+        uint32_t resident = 0;
+        TRY(batch_msm_g1_resident(c > 16 ? 4 : 2, &resident));
+        pk->g1.item_len[2] = fit_item_len(msm1, pk->W, resident);
+    }
     TRY(finish_plan(pk->g1, msm1, pk->W));
     TRY(finish_plan(pk->g1_lat, msm1_lat, pk->W));
     TRY(finish_plan(pk->g2, msm2, pk->W));

@@ -364,7 +364,8 @@ struct ProofConsts {
     G1Affine b0;        // beta_g1 + b_g1_query[0]
     G2Affine b2;        // beta_g2 + b_g2_query[0]
 };
-// g1[q * P + p]: q = 0 A-sum (incl. r*delta), 1 B1-sum (incl. s*delta), 2 L-sum (incl. -rs*delta), 3 H-sum.
+// g1[q * P + p]: q = 0 A-sum (incl. r*delta), 1 B1-sum (incl. s*delta), 2 L-sum (incl. -rs*delta), 3 H-sum,
+// 4 the terms the A and B1 sums share (variables whose A and B1 query points are the same point): A = q0 + q4, B1 = q1 + q4.
 // The stage is a chain of dependent field products per proof (two variable-base scalar multiplications,
 // three inversions), so it is latency-bound.  Its independent strands run on six warps of the CTA
 // (warp-uniform roles, lane = proof) and meet once in shared memory; each scalar multiplication is split by
@@ -397,11 +398,13 @@ __global__ void __launch_bounds__(128) k_assemble(const G1XYZZ *g1, const G2XYZZ
     if (live) {
         if (role <= 1) {
             A = ld_vec(g1 + p);
+            A.add_cold(ld_vec(g1 + 4 * (size_t)P + p));
             A.madd_cold(K.a0);
             if (role == 0) acc = glv_half(A, ld_vec(s + p), 0);
             else st_vec(sm + lane, glv_half(A, ld_vec(s + p), 1));
         } else {
             G1XYZZ B1 = ld_vec(g1 + (size_t)P + p);
+            B1.add_cold(ld_vec(g1 + 4 * (size_t)P + p));
             B1.madd_cold(K.b0);
             st_vec(sm + (role - 1) * 32 + lane, glv_half(B1, ld_vec(r + p), role - 2));
         }

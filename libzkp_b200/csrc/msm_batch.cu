@@ -1,6 +1,7 @@
 // msm_batch.cu — the five MSMs of a batch of proofs as fixed-base table gathers + XYZZ mixed adds
 // (SURVEY.md §8a rows a8-a12; replaces VariableBaseMSM::msm_bigint inside ark-groth16's prover,
 // reached from src/backend/snark.rs:364 and :442).
+#include <algorithm>
 #include <cstdlib>
 #include "tables.h"
 #include "dev_util.cuh"
@@ -127,6 +128,17 @@ uint32_t small_batch_limit() {
         return e ? (uint32_t)atoi(e) : 512u;     // measured crossover on B200: equal at 512 proofs, 12 % slower at 1024
     }();
     return v;
+}
+
+// CTAs of the large-batch G1 gather kernel (128 threads) resident on the whole device at once
+int batch_msm_g1_resident(uint32_t dig_bytes, uint32_t *out) {
+    int dev = 0, sms = 0, per_sm = 0;
+    CUDA_TRY(cudaGetDevice(&dev));
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    if (dig_bytes == 2) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_msm_batch<Fq, 128, int16_t>, 128, 0));
+    else CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_msm_batch<Fq, 128, int32_t>, 128, 0));
+    *out = (uint32_t)std::max(1, sms * per_sm);
+    return LZKP_OK;
 }
 
 // gather + accumulate the items [item0, item0 + count) (partial sums land at their global item index)

@@ -29,6 +29,8 @@ void batch_msm_g1(const BatchMsmArgs &a, cudaStream_t st);
 void batch_msm_g1_items(const BatchMsmArgs &a, uint32_t item0, uint32_t count, cudaStream_t st);
 void batch_msm_g1_reduce(const BatchMsmArgs &a, cudaStream_t st);
 void batch_msm_g2(const BatchMsmArgs &a, cudaStream_t st);
+// CTAs of batch_msm_g1's large-batch gather kernel resident on the current device at once
+int batch_msm_g1_resident(uint32_t dig_bytes, uint32_t *out);
 // Calls of at most this many proofs take the latency-oriented shape (8-unit items, 32-thread CTAs, tree reduction);
 // LZKP_SMALL_BATCH overrides the default for experiments.
 uint32_t small_batch_limit();
