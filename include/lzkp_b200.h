@@ -243,8 +243,10 @@ int lzkp_ntt_device(void *d_in, void *d_out, uint32_t log_n, int inverse, int co
  * set[64], is_real[64]], snark.rs:398,482-492); ok_out[i] = 1 accept, 0 reject (malformed, off-curve, outside the
  * subgroup, non-canonical, wrong input count, or failing the pairing equation).  lzkp_vk_load validates every point
  * of the key (curve and subgroup), as deserialize_uncompressed does, and prepares what ark-groth16 keeps in a
- * PreparedVerifyingKey (line coefficients of -gamma, -delta, beta) plus fixed-base tables for the public-input
- * combination (keys of up to 256 public inputs; 67 MB for membership's 129).
+ * PreparedVerifyingKey (line coefficients of -gamma, -delta, beta) plus fixed-base byte-window tables for the
+ * public-input combination: (n_pub + 2) x 522 240 B of device memory (0.52 MB per public input; 68.4 MB for membership's
+ * 129 inputs, 1.07 GB for the 2049 of a 1024-slot set) plus 51 KB of prepared lines.  If they cannot be allocated the key
+ * still loads; every call then runs one proof per lane, without the two forms below (lzkp_vk_info reports it).
  * Calls of up to three proofs per SM (LZKP_VERIFY_COOP_MAX, 444 on a B200) give every proof a CTA whose warps and lanes
  * share the pairing's arithmetic (one verification 1.8 ms).
  * Larger calls (LZKP_VERIFY_RLC_MIN) check groups of 64 proofs with one random linear combination
@@ -256,6 +258,9 @@ int lzkp_vk_load(const uint8_t *vk_bytes, size_t len, lzkp_vk **out);
 void lzkp_vk_free(lzkp_vk *vk);
 int lzkp_verify_batch(lzkp_vk *vk, size_t n, const uint8_t *proofs, const uint8_t *public_inputs, size_t n_pub,
                       uint8_t *ok_out);
+/* info[0..4) = n_pub, bytes of the byte-window tables on the device, latency form available (1/0), combined form with
+ * the cooperative check available (1/0) */
+int lzkp_vk_info(const lzkp_vk *vk, uint64_t info[4]);
 
 /* MiMC-5 commitment of a u64 (commit_value_snark), 32 B canonical LE.  Host arithmetic, no device. */
 int lzkp_commit_value_snark(uint64_t value, uint8_t out[32]);

@@ -54,6 +54,7 @@ extern "C" {
                                            status: *mut i32) -> c_int;
     pub fn lzkp_vk_load(vk: *const u8, len: usize, out: *mut *mut lzkp_vk) -> c_int;
     pub fn lzkp_vk_free(vk: *mut lzkp_vk);
+    pub fn lzkp_vk_info(vk: *const lzkp_vk, info: *mut u64) -> c_int;
     pub fn lzkp_verify_batch(vk: *mut lzkp_vk, n: usize, proofs: *const u8, public_inputs: *const u8, n_pub: usize,
                              ok_out: *mut u8) -> c_int;
     pub fn lzkp_commit_value_snark(value: u64, out: *mut u8) -> c_int;

@@ -76,6 +76,7 @@ SIGNATURES = {
     "lzkp_ntt_device": (_int, [_vp, _vp, _u32, _int, _int, _vp]),
     "lzkp_vk_load": (_int, [_vp, _sz, C.POINTER(_vp)]),
     "lzkp_vk_free": (None, [_vp]),
+    "lzkp_vk_info": (_int, [_vp, C.POINTER(_u64)]),
     "lzkp_verify_batch": (_int, [_vp, _sz, _vp, _vp, _sz, _vp]),
     "lzkp_commit_value_snark": (_int, [_u64, _vp]),
 }

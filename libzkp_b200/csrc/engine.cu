@@ -1761,6 +1761,11 @@ int lzkp_vk_load(const uint8_t *vk_bytes, size_t len, lzkp_vk **out) {
     *out = new lzkp_vk{v};
     return LZKP_OK;
 }
+int lzkp_vk_info(const lzkp_vk *vk, uint64_t info[4]) {
+    if (!vk || !info) return fail(LZKP_E_INVALID, "null argument");
+    vk_info(vk->v, info);
+    return LZKP_OK;
+}
 void lzkp_vk_free(lzkp_vk *vk) {
     if (!vk) return;
     if (g_device >= 0) cudaSetDevice(g_device);

@@ -11,6 +11,8 @@
 //     of 64 one cooperative combined check (k_rlc_scalars, k_rlc_inputs2, k_rlc_tail_coop); a failing group is re-verified
 //     proof by proof;
 //   * one proof per lane (k_verify4): keys without the latency form's tables, no OS entropy, large failing ranges.
+// Keys above kCoopScanMax public inputs take the same forms; there vk_x of each proof comes from its own kernel (k_vkx)
+// and the combined form's scalar sums from k_rlc_input_sums.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -102,9 +104,12 @@ __global__ void k_vk_prepare(VkDev *vk) {
 // against one thread per proof: 22 vs 39 ms for a single proof, 128 k vs 98 k verifies/s at 4096.)
 //   warp 0: A, B (curve checks), Miller(A, B)           warp 2: C, Miller(C, -delta)
 //   warp 1: vk_x, Miller(vk_x, -gamma)                   warp 3: B in the r-torsion subgroup?
+// vkx (keys above kCoopScanMax inputs that have the byte-window tables): vk_x of every proof, computed by k_vkx; warp 1
+// then only checks that the inputs are canonical.
 __global__ void __launch_bounds__(128) k_verify4(const VkDev *__restrict__ vk, const G1Affine *__restrict__ gamma_abc,
                                                  uint32_t n_pub, const uint8_t *__restrict__ proofs,
-                                                 const Fr *__restrict__ inputs, uint32_t n, uint8_t *__restrict__ ok) {
+                                                 const Fr *__restrict__ inputs, const G1Affine *__restrict__ vkx, uint32_t n,
+                                                 uint8_t *__restrict__ ok) {
     extern __shared__ uint4 smem_raw[];
     Fq12 *sf = reinterpret_cast<Fq12 *>(smem_raw);                       // [2][32] Miller values of warps 1, 2
     __shared__ uint8_t sgood[4][32];
@@ -123,16 +128,22 @@ __global__ void __launch_bounds__(128) k_verify4(const VkDev *__restrict__ vk, c
             skip[0] = !good || P[0].is_inf() || Q[0].is_inf();
             multi_miller_loop<1>(f, P, Q, skip);
         } else if (role == 1) {
-            G1XYZZ acc = G1XYZZ::from_affine(ldg_vec(gamma_abc));
             const Fr *x = inputs + (size_t)p * n_pub;
+            if (vkx) {
 #pragma unroll 1
-            for (uint32_t i = 0; i < n_pub; i++) {
-                Fr xi = ld_vec(x + i);
-                if (!fr_is_canonical(xi)) { good = false; continue; }
-                if (xi.is_zero()) continue;
-                acc.add_cold(scalar_mul(G1XYZZ::from_affine(ldg_vec(gamma_abc + 1 + i)), xi));
+                for (uint32_t i = 0; i < n_pub; i++) good = fr_is_canonical(ld_vec(x + i)) && good;
+                P[0] = ld_vec(vkx + p);
+            } else {
+                G1XYZZ acc = G1XYZZ::from_affine(ldg_vec(gamma_abc));
+#pragma unroll 1
+                for (uint32_t i = 0; i < n_pub; i++) {
+                    Fr xi = ld_vec(x + i);
+                    if (!fr_is_canonical(xi)) { good = false; continue; }
+                    if (xi.is_zero()) continue;
+                    acc.add_cold(scalar_mul(G1XYZZ::from_affine(ldg_vec(gamma_abc + 1 + i)), xi));
+                }
+                P[0] = acc.to_affine();
             }
-            P[0] = acc.to_affine();
             Q[0] = vk->gamma_neg;
             skip[0] = !good || P[0].is_inf() || Q[0].is_inf();
             multi_miller_loop<1>(f, P, Q, skip);
@@ -187,6 +198,7 @@ __device__ __forceinline__ Fr warp_sum_fr(Fr v) {
     return v;
 }
 
+// sx_out == nullptr (keys above kCoopScanMax inputs): no scalar sums here, k_rlc_input_sums forms them per (group, input).
 // Four role warps per 32 proofs, lane = proof, balanced so that the longest strand is ~2200 Fq2 products (a single warp
 // running rho * A and the whole Miller loop was ~3400):
 //   warp 0: A, rho * A -> shared; upper share of Miller(rho A, B), then its 41 squarings; at the end upper * lower
@@ -270,6 +282,7 @@ __global__ void __launch_bounds__(128) k_rlc_prepare(const VkDev *__restrict__ v
         ok[p] = good ? 1 : 0;
     } else if (role == 2) {
         if (live) st_vec(rc_out + p, good ? rc : G1XYZZ::inf());
+        if (!sx_out) return;                                                     // k_rlc_input_sums forms the sums
         // sums over this CTA's 32 proofs of rho_p * x_pj, j = 0 .. n_pub (x_p0 = 1), as plain (canonical) residues mod r
         Fr rho_c = Fr::zero(), rho_m = Fr::zero();
         if (good) {
@@ -325,7 +338,7 @@ __global__ void __launch_bounds__(64) k_rlc_prepare_seq(const VkDev *__restrict_
             st_vec(rc_out + p, good ? rc : G1XYZZ::inf());
         }
     }
-    {   // sums over these 32 proofs of rho_p * x_pj, j = 0 .. n_pub (x_p0 = 1), as plain (canonical) residues mod r
+    if (sx_out) {   // sums over these 32 proofs of rho_p * x_pj, j = 0 .. n_pub (x_p0 = 1), as plain (canonical) residues mod r
         Fr rho_c = Fr::zero(), rho_m = Fr::zero();
         if (good) {
             rho_c = glv64_coefficient(k);
@@ -521,6 +534,7 @@ __device__ __forceinline__ void set_emb(FChain &c, const G1Affine &P) {
 //   warp 2  AB_LOWER: lower share of the (A, B) f chain, then the multiplying side of the three exponentiations by x
 //   warp 6  DELTA:    Miller(C, -delta) on prepared lines                                            (beside warp 2)
 //   warp 3  LADDER:   B in the r-torsion subgroup?                                                    warp 5: idle
+// vkx: keys above kCoopScanMax inputs, whose scan would be the longest strand; k_vkx has computed vk_x of every proof.
 enum CoopRole { kAbUpper = 0, kLines = 1, kAbLower = 2, kLadder = 3, kGamma = 4, kIdle = 5, kDelta = 6 };
 // MIN_CTAS = 1: all the registers the code wants (250; one CTA per SM) for calls of at most one proof per SM; MIN_CTAS = 2: 128
 // registers, two proofs per SM side by side - 10 % slower each (1.99 against 1.80 ms), 1.5x the throughput from 149 proofs on.
@@ -529,7 +543,7 @@ __global__ void __launch_bounds__(kCoopThreads, MIN_CTAS) k_verify_coop(const Vk
                                                               const G1Affine *__restrict__ tab, const Fq2 *__restrict__ lines_gamma,
                                                               const Fq2 *__restrict__ lines_delta, uint32_t n_pub,
                                                               const uint8_t *__restrict__ proofs, const uint8_t *__restrict__ inputs,
-                                                              uint8_t *__restrict__ ok) {
+                                                              const G1Affine *__restrict__ vkx, uint8_t *__restrict__ ok) {
     extern __shared__ uint4 smem_raw[];
     CoopSmem &sm = *reinterpret_cast<CoopSmem *>(smem_raw);
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31, p = blockIdx.x;
@@ -569,7 +583,7 @@ __global__ void __launch_bounds__(kCoopThreads, MIN_CTAS) k_verify_coop(const Vk
         FChain &c = sm.fc[1];
         bool skip = true;
         if (all_good) {
-            const G1Affine P = coop::vkx_from_tables(tab, gamma_abc, x, n_pub);
+            const G1Affine P = vkx ? ld_vec(vkx + p) : coop::vkx_from_tables(tab, gamma_abc, x, n_pub);
             skip = P.is_inf() || vk->gamma_neg.is_inf();
             if (!skip) set_emb(c, P);
         }
@@ -707,6 +721,38 @@ __global__ void __launch_bounds__(128) k_rlc_scalars(const Fr *__restrict__ sx_i
     for (uint32_t b = cta_lo; b < cta_hi; b++) sum = sum + ld_vec(sx_in + (size_t)b * (n_pub + 1) + j);
     st_vec(gS + t, sum);
 }
+// gS[g][j] straight from the inputs, thread = (group g, column j): keys above kCoopScanMax inputs.  There the scalar sums of
+// k_rlc_prepare are one warp walking all n_pub columns per 32 proofs (a shuffle tree per column) beside the Miller loop;
+// here the group's 64 coefficients are formed once in shared memory and every thread sums 64 products of one column.
+// ok[p] (k_rlc_prepare's verdict on the proof's form) decides whether rho_p takes part, as `good` does there.
+__global__ void __launch_bounds__(128) k_rlc_input_sums(const Fr *__restrict__ inputs, const uint32_t *__restrict__ rho,
+                                                        const uint8_t *__restrict__ ok, uint32_t n, uint32_t n_pub,
+                                                        Fr *__restrict__ gS) {
+    __shared__ Fr s_c[kRlcGroup], s_m[kRlcGroup];          // rho_p canonical / as a Montgomery residue; zero if malformed
+    const uint32_t g = blockIdx.x, j = blockIdx.y * blockDim.x + threadIdx.x, lo = g * kRlcGroup, cnt = min(n - lo, kRlcGroup);
+    if (threadIdx.x < cnt) {
+        const uint32_t p = lo + threadIdx.x;
+        Fr c = Fr::zero();
+        if (ok[p]) {
+            const uint4 r4 = reinterpret_cast<const uint4 *>(rho)[p];
+            uint32_t k[4] = {r4.x, r4.y, r4.z, r4.w};
+            c = glv64_coefficient(k);
+        }
+        st_vec(s_c + threadIdx.x, c);
+        st_vec(s_m + threadIdx.x, Fr::from_canonical(c));
+    }
+    __syncthreads();
+    if (j > n_pub) return;
+    Fr sum = Fr::zero();
+    if (j == 0) {
+        for (uint32_t q = 0; q < cnt; q++) sum = sum + ld_vec(s_c + q);
+    } else {
+        const Fr *x = inputs + (size_t)lo * n_pub + (j - 1);
+#pragma unroll 4
+        for (uint32_t q = 0; q < cnt; q++) sum = sum + ld_vec(s_m + q) * ld_vec(x + (size_t)q * n_pub);
+    }
+    st_vec(gS + (size_t)g * (n_pub + 1) + j, sum);
+}
 // X[g][j] = S[g][j] * gamma_abc[j] for j <= n_pub, and the extra column X[g][n_pub + 1] = S[g][0] * alpha, from the byte-window
 // tables: one warp per (g, j), lane = byte of the scalar, then a shuffle tree.  (As a 254-bit scalar multiplication on one
 // thread per (g, j) this stage was a 1.4 ms chain in EVERY combined-form call, whatever its size.)
@@ -729,6 +775,57 @@ __global__ void __launch_bounds__(128) k_rlc_inputs2(const Fr *__restrict__ gS, 
         acc.add_cold(o);
     }
     if (lane == 0) st_vec(gX + t, acc);
+}
+
+// ---- vk_x of every proof of a call, keys above kCoopScanMax public inputs.  The latency form's GAMMA warp scans all
+// n_pub x 32 (input, byte) pairs itself (coop::vkx_from_tables), and the Miller loop against -gamma waits for it: at 2049
+// inputs that is ~2000 steps on the critical path.  Here one CTA per proof: warp w takes the slices w, w + warps, ... of
+// `slice` inputs; a lane holds one input (32 bytes in registers) and walks its bytes upwards, with a ballot skipping the
+// windows where no lane of the warp has a nonzero byte and ending the chunk once no lane has one left (64-bit values: 8
+// windows, bits: 1).  Partial XYZZ sums, gamma_abc[0] on warp 0, one shuffle-tree reduction, affine result in vkx[p].
+constexpr uint32_t kCoopScanMax = 256;       // keys of up to this many inputs keep the in-kernel scan
+constexpr uint32_t kVkxWarps = 8;
+// Inputs per slice.  At 2049 inputs (B200, 1000 W) k_vkx takes 0.22 / 0.49 / 1.07 ms for 1 / 64 / 444 proofs with slices of 64;
+// 32 and 128 tie at 1 and 64 proofs and lose at 444 (1.16, 1.18 ms), 256 and 512 lose at 64 proofs (0.57, 0.83 ms).
+constexpr uint32_t kVkxSlice = 64;
+__global__ void __launch_bounds__(kVkxWarps * 32) k_vkx(const G1Affine *__restrict__ tab, const G1Affine *__restrict__ gamma_abc,
+                                                        uint32_t n_pub, uint32_t slice, const uint8_t *__restrict__ inputs,
+                                                        G1Affine *__restrict__ vkx) {
+    __shared__ G1XYZZ part[kVkxWarps * 32];
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31, warps = blockDim.x >> 5, p = blockIdx.x;
+    const uint4 *x = reinterpret_cast<const uint4 *>(inputs + (size_t)p * n_pub * 32);
+    G1XYZZ acc = G1XYZZ::inf();
+    if (threadIdx.x == 0) acc = G1XYZZ::from_affine(ldg_vec(gamma_abc));
+#pragma unroll 1
+    for (uint32_t s0 = warp * slice; s0 < n_pub; s0 += warps * slice) {
+        const uint32_t end = min(n_pub, s0 + slice);
+#pragma unroll 1
+        for (uint32_t c = s0; c < end; c += 32) {
+            const uint32_t i = c + lane;
+            uint32_t v[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+            if (i < end) {
+                const uint4 lo = __ldg(x + 2 * (size_t)i), hi = __ldg(x + 2 * (size_t)i + 1);
+                v[0] = lo.x; v[1] = lo.y; v[2] = lo.z; v[3] = lo.w; v[4] = hi.x; v[5] = hi.y; v[6] = hi.z; v[7] = hi.w;
+            }
+            const G1Affine *row = tab + (size_t)i * coop::kTabWindows * coop::kTabDigits;
+#pragma unroll 1
+            for (uint32_t w = 0; w < coop::kTabWindows; w++) {
+                const uint32_t rest = v[0] | v[1] | v[2] | v[3] | v[4] | v[5] | v[6] | v[7];
+                if (__ballot_sync(0xffffffffu, rest != 0) == 0) break;
+                const uint32_t d = v[0] & 0xFFu;
+                if (d) acc.madd(ldg_vec(row + w * coop::kTabDigits + (d - 1)));
+#pragma unroll
+                for (int k = 0; k < 7; k++) v[k] = __funnelshift_r(v[k], v[k + 1], 8);
+                v[7] >>= 8;
+            }
+        }
+    }
+    st_vec(part + threadIdx.x, acc);
+    __syncthreads();
+    if (warp == 0) {
+        const G1Affine r = coop_sum_g1(part, blockDim.x);
+        if (lane == 0) st_vec(vkx + p, r);
+    }
 }
 
 // LZKP_COOP_SELFTEST=1 at key load: the cooperative Miller loop (both line sources), final exponentiation and subgroup
@@ -844,24 +941,32 @@ struct VerifyingKeyDev {
     DBuf d_p, d_x, d_ok;          // grow-only staging of a batch (calls on one key serialize on mu)
     DBuf d_rho, d_f, d_rc, d_sx, d_gF, d_gC, d_gS, d_gX, d_gok;     // random-linear-combination path (large batches)
     DBuf lines_gamma, lines_delta, lines_beta, tab;                             // latency form (coop.cuh): prepared lines, vk_x byte-window tables
+    DBuf d_vkx;                                                                  // vk_x per proof (k_vkx; keys above kCoopScanMax inputs)
     bool coop_ok = false;
     uint32_t n_pub = 0;
     std::mutex mu;
 };
 
-// The latency form's per-key data: prepared lines of -gamma / -delta and the byte-window tables of gamma_abc (67 MB for the
-// 129 inputs of the membership key; keys with more than kCoopMaxInputs inputs keep the lane-per-proof kernel).
-constexpr uint32_t kCoopMaxInputs = 256;
+// The latency and combined forms' per-key data: prepared lines of -gamma / -delta / beta and the byte-window tables of
+// gamma_abc and alpha, (n_pub + 2) x 32 x 255 affine points = 0.52 MB per public input (68.4 MB for the 129 inputs of the
+// membership key, 1.07 GB for the 2049 of membership with 1024 slots).  When they cannot be allocated the key still loads
+// and verifies one proof per lane (k_verify4).
+static size_t coop_table_bytes(uint32_t n_pub) {
+    return (size_t)(n_pub + 2) * coop::kTabWindows * coop::kTabDigits * sizeof(G1Affine);
+}
 static int coop_prepare(VerifyingKeyDev *V) {
-    if (V->n_pub > kCoopMaxInputs) return LZKP_OK;
     const size_t line_bytes = (size_t)coop::kLines * 3 * sizeof(Fq2);
-    TRY(V->lines_gamma.alloc(line_bytes)); TRY(V->lines_delta.alloc(line_bytes)); TRY(V->lines_beta.alloc(line_bytes));
+    if (V->lines_gamma.alloc(line_bytes) != LZKP_OK || V->lines_delta.alloc(line_bytes) != LZKP_OK ||
+        V->lines_beta.alloc(line_bytes) != LZKP_OK || V->tab.alloc(coop_table_bytes(V->n_pub)) != LZKP_OK) {
+        V->lines_gamma.release(); V->lines_delta.release(); V->lines_beta.release(); V->tab.release();
+        cudaGetLastError();
+        return LZKP_OK;                                                          // coop_ok stays false
+    }
     CUDA_TRY(cudaMemset(V->lines_gamma.p, 0, line_bytes)); CUDA_TRY(cudaMemset(V->lines_delta.p, 0, line_bytes));
     CUDA_TRY(cudaMemset(V->lines_beta.p, 0, line_bytes));
     LAUNCH(k_prepare_lines, 1, 32, 0, 0, V->vk.as<VkDev>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(), V->lines_beta.as<Fq2>());
     {
         const uint32_t threads = (V->n_pub + 2) * coop::kTabWindows;
-        TRY(V->tab.alloc((size_t)threads * coop::kTabDigits * sizeof(G1Affine)));
         LAUNCH(k_vk_tables, (threads + 63) / 64, 64, 0, 0, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(), V->n_pub, V->tab.as<G1Affine>());
     }
     CUDA_TRY(cudaDeviceSynchronize());
@@ -955,6 +1060,12 @@ int vk_load(const uint8_t *bytes, size_t len, VerifyingKeyDev **out) {
 }
 void vk_free(VerifyingKeyDev *V) { delete V; }
 uint32_t vk_num_inputs(const VerifyingKeyDev *V) { return V->n_pub; }
+void vk_info(const VerifyingKeyDev *V, uint64_t info[4]) {
+    info[0] = V->n_pub;
+    info[1] = V->coop_ok ? V->tab.bytes : 0;     // (n_pub + 2) x 32 x 255 x 64 B; the prepared lines add 3 x 17 KB
+    info[2] = V->coop_ok ? 1 : 0;          // the latency form (one proof per CTA)
+    info[3] = V->coop_ok ? 1 : 0;          // the combined form with the cooperative check from 3 x SMs + 1 proofs
+}
 
 int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint8_t *inputs, size_t n_pub, uint8_t *ok_out) {
     std::lock_guard<std::mutex> lk(V->mu);
@@ -974,20 +1085,30 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
     int sm_count = 148;
     cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, current_device() < 0 ? 0 : current_device());
     const size_t coop_max = getenv("LZKP_VERIFY_COOP_MAX") ? (size_t)atoll(getenv("LZKP_VERIFY_COOP_MAX")) : (size_t)3 * sm_count;
+    // Keys above kCoopScanMax inputs: vk_x of the proofs of a range comes from k_vkx, for the latency form and k_verify4 alike.
+    const bool vkx_kernel = V->coop_ok && n_pub > kCoopScanMax;
+    if (vkx_kernel) TRY(V->d_vkx.ensure(n * sizeof(G1Affine)));
     auto verify_range = [&](size_t off, size_t cnt) {             // independent verification of proofs [off, off + cnt)
+        const G1Affine *vkx = nullptr;
+        if (vkx_kernel) {
+            const uint32_t warps = std::min<uint32_t>(kVkxWarps, ((uint32_t)n_pub + kVkxSlice - 1) / kVkxSlice);
+            LAUNCH(k_vkx, (unsigned)cnt, warps * 32, 0, 0, V->tab.as<G1Affine>(), V->gamma_abc.as<G1Affine>(), (uint32_t)n_pub, kVkxSlice,
+                   d_x.as<uint8_t>() + off * n_pub * 32, V->d_vkx.as<G1Affine>() + off);
+            vkx = V->d_vkx.as<G1Affine>() + off;
+        }
         if (V->coop_ok && cnt <= coop_max) {
             if (cnt <= (size_t)sm_count)
                 LAUNCH(k_verify_coop<1>, (unsigned)cnt, kCoopThreads, sizeof(CoopSmem), 0, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
                        V->tab.as<G1Affine>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(), (uint32_t)n_pub,
-                       d_p.as<uint8_t>() + off * 256, d_x.as<uint8_t>() + off * n_pub * 32, d_ok.as<uint8_t>() + off);
+                       d_p.as<uint8_t>() + off * 256, d_x.as<uint8_t>() + off * n_pub * 32, vkx, d_ok.as<uint8_t>() + off);
             else
                 LAUNCH(k_verify_coop<2>, (unsigned)cnt, kCoopThreads, sizeof(CoopSmem), 0, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
                        V->tab.as<G1Affine>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(), (uint32_t)n_pub,
-                       d_p.as<uint8_t>() + off * 256, d_x.as<uint8_t>() + off * n_pub * 32, d_ok.as<uint8_t>() + off);
+                       d_p.as<uint8_t>() + off * 256, d_x.as<uint8_t>() + off * n_pub * 32, vkx, d_ok.as<uint8_t>() + off);
             return;
         }
         LAUNCH(k_verify4, (unsigned)((cnt + 31) / 32), 128, 64 * sizeof(Fq12), 0, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
-               (uint32_t)n_pub, d_p.as<uint8_t>() + off * 256, d_x.as<Fr>() + off * n_pub, (uint32_t)cnt, d_ok.as<uint8_t>() + off);
+               (uint32_t)n_pub, d_p.as<uint8_t>() + off * 256, d_x.as<Fr>() + off * n_pub, vkx, (uint32_t)cnt, d_ok.as<uint8_t>() + off);
     };
     // Above the latency form's range the random-linear-combination form takes over: 2.4x less work per proof (one Miller
     // loop instead of three, one final exponentiation per 64 proofs) and, with the cooperative combined check, a short
@@ -1024,7 +1145,12 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
         }
     }
     TRY(V->d_rho.ensure(n * 16)); TRY(V->d_f.ensure(n * sizeof(Fq12))); TRY(V->d_rc.ensure(n * sizeof(G1XYZZ)));
-    TRY(V->d_sx.ensure((size_t)ctas * np1 * sizeof(Fr)));
+    static const bool tail_lanes = getenv("LZKP_RLC_TAIL_LANES") != nullptr;      // A/B switch: the lane-per-group tail
+    // Keys above kCoopScanMax inputs: the scalar sums per (group, input) in k_rlc_input_sums, not in the per-proof kernel.  At
+    // 2049 inputs (B200, 1000 W) the per-proof kernel's sums strand outlasts its Miller loop: k_rlc_prepare 5.83 against
+    // 3.97 ms at 445 proofs, 6.89 against 4.12 at 4096; k_rlc_input_sums itself takes 0.04 / 0.18 ms.
+    const bool input_sums = V->coop_ok && !tail_lanes && n_pub > kCoopScanMax;
+    if (!input_sums) TRY(V->d_sx.ensure((size_t)ctas * np1 * sizeof(Fr)));
     TRY(V->d_gF.ensure((size_t)groups * sizeof(Fq12))); TRY(V->d_gC.ensure((size_t)groups * sizeof(G1XYZZ)));
     TRY(V->d_gS.ensure((size_t)groups * np1 * sizeof(Fr))); TRY(V->d_gX.ensure((size_t)groups * (np1 + 1) * sizeof(G1XYZZ)));
     TRY(V->d_gok.ensure(groups));
@@ -1040,15 +1166,19 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
     // (a 128-register build of the role kernel, four CTAs per SM, for calls of up to two of these waves: 15.0 - 19.0 ms against
     // 13.3 - 13.7 ms for the sequential kernel at 12 288 - 18 944 proofs - rejected)
     const bool prep_roles = force ? atoi(force) != 0 : n <= (size_t)sm_count * 2 * 32;
+    Fr *sx = input_sums ? nullptr : V->d_sx.as<Fr>();
     if (prep_roles)
         LAUNCH(k_rlc_prepare, ctas, 128, 32 * (sizeof(Fq12) + sizeof(G1Affine)), 0, V->vk.as<VkDev>(), (uint32_t)n_pub, d_p.as<uint8_t>(), d_x.as<Fr>(), V->d_rho.as<uint32_t>(),
-               (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), V->d_sx.as<Fr>(), d_ok.as<uint8_t>());
+               (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), sx, d_ok.as<uint8_t>());
     else
         LAUNCH(k_rlc_prepare_seq, (ctas + 1) / 2, 64, 0, 0, V->vk.as<VkDev>(), (uint32_t)n_pub, d_p.as<uint8_t>(), d_x.as<Fr>(),
-               V->d_rho.as<uint32_t>(), (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), V->d_sx.as<Fr>(), d_ok.as<uint8_t>());
-    static const bool tail_lanes = getenv("LZKP_RLC_TAIL_LANES") != nullptr;      // A/B switch: the lane-per-group tail
+               V->d_rho.as<uint32_t>(), (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), sx, d_ok.as<uint8_t>());
     if (V->coop_ok && !tail_lanes) {
-        LAUNCH(k_rlc_scalars, (groups * np1 + 127) / 128, 128, 0, 0, V->d_sx.as<Fr>(), (uint32_t)n, (uint32_t)n_pub, groups, V->d_gS.as<Fr>());
+        if (input_sums)
+            LAUNCH(k_rlc_input_sums, dim3(groups, (np1 + 127) / 128), 128, 0, 0, d_x.as<Fr>(), V->d_rho.as<uint32_t>(), d_ok.as<uint8_t>(),
+                   (uint32_t)n, (uint32_t)n_pub, V->d_gS.as<Fr>());
+        else
+            LAUNCH(k_rlc_scalars, (groups * np1 + 127) / 128, 128, 0, 0, V->d_sx.as<Fr>(), (uint32_t)n, (uint32_t)n_pub, groups, V->d_gS.as<Fr>());
         LAUNCH(k_rlc_inputs2, (groups * (np1 + 1) + 3) / 4, 128, 0, 0, V->d_gS.as<Fr>(), V->tab.as<G1Affine>(), (uint32_t)n_pub, groups,
                V->d_gX.as<G1XYZZ>());
         if (groups <= 2u * (uint32_t)sm_count)

@@ -9,6 +9,7 @@ struct VerifyingKeyDev;
 int vk_load(const uint8_t *bytes, size_t len, VerifyingKeyDev **out);
 void vk_free(VerifyingKeyDev *v);
 uint32_t vk_num_inputs(const VerifyingKeyDev *v);
+void vk_info(const VerifyingKeyDev *v, uint64_t info[4]);
 int verify_batch(VerifyingKeyDev *v, size_t n, const uint8_t *proofs, const uint8_t *inputs, size_t n_pub, uint8_t *ok_out);
 }  // namespace eng
 }  // namespace lzkp

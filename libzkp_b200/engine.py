@@ -383,6 +383,12 @@ class VerifyingKey:
         check(lib().lzkp_verify_batch(self._h, n, _p(proofs), _p(x) if x.size else None, n_pub, _p(ok)))
         return ok.astype(bool)
 
+    def info(self):
+        """(n_pub, table bytes, latency form available, combined form available) of the loaded key."""
+        v = (C.c_uint64 * 4)()
+        check(lib().lzkp_vk_info(self._h, v))
+        return int(v[0]), int(v[1]), bool(v[2]), bool(v[3])
+
     def close(self):
         if self._h:
             lib().lzkp_vk_free(self._h)
