@@ -80,6 +80,31 @@ struct XYZZ {
         zz = zz * PP;
         zzz = zzz * PPP;
     }
+    // madd with the accumulator in field.cuh's redundant form (F = Fq): x, y, zz, zzz in [0, 2p), p canonical.  The
+    // same formula and residues as madd without the final subtraction of each product; canonical() brings the result
+    // back.  The zero tests compare residues (0 or p), not bit patterns.
+    // Bounds in multiples of p (R = 2^256 = 5.29p; a lazy product is < a b / R + p):
+    LZ_HD void madd_lazy(const Affine<F> &p) {
+        if (p.is_inf()) return;
+        if (zz.is_zero_2p()) { *this = from_affine(p); return; }
+        F U2 = F::mul_lazy(p.x, zz), S2 = F::mul_lazy(p.y, zzz);     // 1 x 2: < 1.38
+        F Pp = F::sub_2p(U2, x), R = F::sub_2p(S2, y);               // [0, 2)
+        if (Pp.is_zero_2p()) {
+            if (R.is_zero_2p()) *this = dbl_affine(p);
+            else *this = inf();
+            return;
+        }
+        F PP = Pp.sqr_lazy();                                        // 2 x 2: < 1.76
+        F PPP = F::mul_lazy(Pp, PP), Q = F::mul_lazy(x, PP);         // 2 x 1.76: < 1.67
+        F RR = R.sqr_lazy();                                         // < 1.76
+        F X3 = F::sub_2p(F::sub_2p(RR, PPP), F::add_2p(Q, Q));       // [0, 2) from operands < 2
+        F Y3 = F::msub_lazy(R, F::sub_2p(Q, X3), y, PPP);            // all four < 2: < 2
+        x = X3; y = Y3;
+        zz = F::mul_lazy(zz, PP);                                    // 2 x 1.76: < 1.67
+        zzz = F::mul_lazy(zzz, PPP);                                 // 2 x 1.67: < 1.63
+    }
+    // [0, 2p) coordinates -> canonical
+    LZ_HD XYZZ canonical() const { return XYZZ{x.canonical(), y.canonical(), zz.canonical(), zzz.canonical()}; }
     // *this += q   (add-2008-s): 12M + 2S
     LZ_HD void add(const XYZZ &q) {
         if (q.is_inf()) return;

@@ -3,7 +3,8 @@
 // Replaces what ark-ff's Fp256<MontBackend<_,4>> does for the reference's prover
 // (reference call sites: src/backend/snark.rs:194,203-208 and everything inside
 // Groth16::prove at snark.rs:364,442).  Same field, same Montgomery radix R = 2^256,
-// values always fully reduced, so canonical outputs are bit-identical.
+// values fully reduced, so canonical outputs are bit-identical.  (The G1 gather kernel's
+// accumulator alone runs in a redundant form, [0, 2p), and is reduced before it is stored.)
 //
 // Multiplication is a CIOS Montgomery product built from carry-chained
 // mad.lo.cc / madc.hi.cc rows; ptxas fuses each lo/hi pair into one
@@ -594,7 +595,23 @@ struct alignas(16) Fp {
     LZ_HD Fp dbl() const { return *this + *this; }
 
     // Montgomery product a*b*R^-1 mod p.
-    LZ_HD friend Fp operator*(const Fp &a, const Fp &b) {
+    LZ_HD friend Fp operator*(const Fp &a, const Fp &b) { return reduce_once(mul_lazy(a, b).l); }
+    LZ_HD Fp sqr() const { return reduce_once(sqr_lazy().l); }
+    // Montgomery reduction of a 16-limb T < p * 2^256, canonical result.
+    LZ_HD static Fp reduce_wide(const uint32_t (&T)[16]) { return reduce_once(reduce_wide_lazy(T).l); }
+    // a*b - c*d with ONE reduction (the Y3 of every XYZZ formula), a, b, c, d < p.  200 multiply-adds instead of 272.
+    LZ_HD static Fp msub(const Fp &a, const Fp &b, const Fp &c, const Fp &d) { return reduce_once(msub_lazy(a, b, c, d).l); }
+
+    // ---- Redundant form: values in [0, 2p) instead of [0, p), for the G1 table-gather kernel's mixed addition
+    // (ec.cuh madd_lazy).  The primitives below are the cores of the canonical operations without their final
+    // conditional subtraction (8 subtractions + 8 selects each).  BN254's p = 0.18903 R (R = 2^256), so 4p < R and
+    // the Montgomery reduction still returns below 2p from operands below 2p: the bound of every result is stated
+    // beside it.  Units below: multiples of p, with R = 5.29 p.
+    //
+    // CIOS product without the final subtraction: (a b + m p) / R < a b / R + p for any a < R - p (the accumulator,
+    // at most (a + p) 2^32 before each shift, stays below 2^288) and any b < R.  a, b < 2p: < 1.76p; a < p, b < 2p:
+    // < 1.38p; generally < 2p whenever a b < p R.
+    LZ_HD static Fp mul_lazy(const Fp &a, const Fp &b) {
         uint32_t X[8], Y[8];      // aligned / offset accumulators (roles swap every iteration)
         uint32_t m, c;
         // i = 0
@@ -626,27 +643,30 @@ struct alignas(16) Fp {
             }
         }
         // After i = 7 (odd): Y aligned with Y[0] == 0, X offset.  result = X + (Y >> 32).
-        uint32_t hi[8], s[8];
+        uint32_t hi[8];
 #pragma unroll
         for (int j = 0; j < 7; j++) hi[j] = Y[j + 1];
         hi[7] = 0;
-        add8(s, X, hi);
-        return reduce_once(s);
+        Fp s;
+        add8(s.l, X, hi);
+        return s;
     }
     // a^2 * R^-1 by column scanning with the reduction interleaved (FIPS): 36 + 64 limb products instead of 64 + 64.
     //   a^2 = sum_i a_i B^i * (a_i B^i + 2 * (a div B^(i+1)) * B^(i+1)):  row i multiplies a_i by a_i, by
     //   e_(i+1) = 2 a_(i+1) mod 2^32 (bit 0 clear) and by d_j = limb j of 2a (j > i + 1); 2a < 2^256 because a < 2^255.
     // Measured 79 G squarings/s against 64 G products/s (tools/microbench/mulcs.cu), bit-exact against operator*.
-    LZ_HD Fp sqr() const {
+    // Without the final subtraction: a < 2^255 (= 2.64p), result < a^2 / R + p; a < 2p: < 1.76p.
+    LZ_HD Fp sqr_lazy() const {
 #ifdef LZKP_SQR_AS_MUL           // A/B switch: the round-1 behaviour (a full product)
-        return *this * *this;
+        return mul_lazy(*this, *this);
 #endif
         uint32_t d[8], e[8];
         d[0] = l[0] << 1;
         e[0] = 0;
 #pragma unroll
         for (int i = 1; i < 8; i++) { d[i] = (l[i] << 1) | (l[i - 1] >> 31); e[i] = l[i] << 1; }
-        uint32_t t0 = 0, t1 = 0, t2 = 0, m[8], r[8];
+        uint32_t t0 = 0, t1 = 0, t2 = 0, m[8];
+        Fp r;
 #pragma unroll
         for (int k = 0; k < 15; k++) {
 #pragma unroll
@@ -665,17 +685,17 @@ struct alignas(16) Fp {
             } else {
 #pragma unroll
                 for (int i = k - 7; i < 8; i++) mac3(t0, t1, t2, m[i], P::MOD(k - i));
-                r[k - 8] = t0;
+                r.l[k - 8] = t0;
             }
             t0 = t1; t1 = t2; t2 = 0;
         }
-        r[7] = t0;
-        return reduce_once(r);
+        r.l[7] = t0;
+        return r;
     }
-    // Montgomery reduction of a 16-limb T < p * 2^256: T * R^-1 mod p = (T_lo + M p) / R + T_hi, where the eight
-    // rounds run on the lower half alone (U = (T_lo + M p) / R <= p) in the product's aligned / offset accumulators,
-    // and T_hi < p joins at the end: U + T_hi < 2p.
-    LZ_HD static Fp reduce_wide(const uint32_t (&T)[16]) {
+    // Montgomery reduction of a 16-limb T < p * 2^256 without the final subtraction: T * R^-1 mod p =
+    // (T_lo + M p) / R + T_hi, where the eight rounds run on the lower half alone (U = (T_lo + M p) / R <= p) in the
+    // product's aligned / offset accumulators, and T_hi < p joins at the end: U + T_hi < 2p.
+    LZ_HD static Fp reduce_wide_lazy(const uint32_t (&T)[16]) {
         uint32_t X[8], Y[8];
         uint32_t m, c;
 #pragma unroll
@@ -697,25 +717,61 @@ struct alignas(16) Fp {
             }
         }
         // after i = 7: Y aligned with Y[0] == 0, X offset: U = X + (Y >> 32)
-        uint32_t hi[8], th[8], u[8], s_[8];
+        uint32_t hi[8], th[8], u[8];
 #pragma unroll
         for (int j = 0; j < 7; j++) hi[j] = Y[j + 1];
         hi[7] = 0;
 #pragma unroll
         for (int j = 0; j < 8; j++) th[j] = T[8 + j];
         add8(u, X, hi);
-        add8(s_, u, th);
-        return reduce_once(s_);
+        Fp s_;
+        add8(s_.l, u, th);
+        return s_;
     }
-    // a*b - c*d with ONE reduction (the Y3 of every XYZZ formula): two 16-limb products, the difference brought back
-    // into [0, p * 2^256) by adding p * 2^256 when negative.  200 multiply-adds instead of 272.
-    LZ_HD static Fp msub(const Fp &a, const Fp &b, const Fp &c, const Fp &d) {
+    // a*b - c*d as two 16-limb products, the difference brought back into [0, p * 2^256) by adding p * 2^256 when
+    // negative, and one reduction without the final subtraction.  a b < p R and c d < p R (all four below 2p: 4p^2 =
+    // 0.76 p R): result < 2p.
+    LZ_HD static Fp msub_lazy(const Fp &a, const Fp &b, const Fp &c, const Fp &d) {
         uint32_t t0[16], t1[16];
         mul_wide(t0, a.l, b.l);
         mul_wide(t1, c.l, d.l);
         const uint32_t bw = sub16(t0, t0, t1);
         wide_fix_negative<P>(t0, bw);
-        return reduce_wide(t0);
+        return reduce_wide_lazy(t0);
+    }
+    // a - b, plus 2p when negative:  a, b < 2p -> [0, 2p)
+    LZ_HD static Fp sub_2p(const Fp &a, const Fp &b) {
+        Fp d, e, r;
+        uint32_t bw = sub8(d.l, a.l, b.l);
+        add8(e.l, d.l, modulus2().l);
+#pragma unroll
+        for (int i = 0; i < 8; i++) r.l[i] = bw ? e.l[i] : d.l[i];
+        return r;
+    }
+    // a + b, less 2p when at least 2p:  a, b < 2p -> [0, 2p)
+    LZ_HD static Fp add_2p(const Fp &a, const Fp &b) {
+        uint32_t s[8];
+        Fp d, r;
+        add8(s, a.l, b.l);        // a + b < 4p < 2^256: no carry out
+        uint32_t bw = sub8(d.l, s, modulus2().l);
+#pragma unroll
+        for (int i = 0; i < 8; i++) r.l[i] = bw ? s[i] : d.l[i];
+        return r;
+    }
+    // x == 0 mod p for x < 2p: x is 0 or p
+    LZ_HD bool is_zero_2p() const {
+        uint32_t z = 0, q = 0;
+#pragma unroll
+        for (int i = 0; i < 8; i++) { z |= l[i]; q |= l[i] ^ P::MOD(i); }
+        return z == 0 || q == 0;
+    }
+    // [0, 2p) -> [0, p)
+    LZ_HD Fp canonical() const { return reduce_once(l); }
+    LZ_HD static Fp modulus2() {
+        Fp r;
+#pragma unroll
+        for (int i = 0; i < 8; i++) r.l[i] = (P::MOD(i) << 1) | (i ? P::MOD(i - 1) >> 31 : 0u);
+        return r;
     }
 
     // canonical (plain integer, < p) <-> Montgomery

@@ -30,6 +30,10 @@ __global__ void __launch_bounds__(BLOCK, LZKP_G2_MINB_SEL(F)) k_msm_batch(const 
     const uint32_t p = blockIdx.x * BLOCK + threadIdx.x, item = blockIdx.y;
     if (p >= P) return;
     const uint2 range = items[item];
+    // G1 accumulates in field.cuh's redundant form (madd_lazy: no final subtraction after each product) and is made
+    // canonical before it is stored.  G2 keeps the canonical madd: with the lazy one the kernel spilled 844 B instead
+    // of 308 B at its 168 registers.
+    constexpr bool lazy = sizeof(F) == sizeof(Fq);
     XYZZ<F> acc = XYZZ<F>::inf();
     // Software pipeline: the table point of unit u+1 is in flight under the add of unit u.  (Also keeping the digit of
     // unit u+2 in flight gained 2 % with 4-byte digits at 156 registers, but costs the fourth resident CTA: dropped.)
@@ -43,10 +47,14 @@ __global__ void __launch_bounds__(BLOCK, LZKP_G2_MINB_SEL(F)) k_msm_batch(const 
             dn = dig[(size_t)__ldg(unit_dig + u + 1) * P + p];
             if (dn) ptn = gather_point(table, N, __ldg(unit_tbl + u + 1), dn);
         }
-        if (d) acc.madd(pt);
+        if (d) {
+            if constexpr (lazy) acc.madd_lazy(pt);
+            else acc.madd(pt);
+        }
         d = dn;
         pt = ptn;
     }
+    if constexpr (lazy) acc = acc.canonical();
     st_vec(partial + (size_t)item * P + p, acc);
 }
 // Reduction of the per-item partial sums, in two launches so that the serial chain per thread stays short:
