@@ -258,6 +258,21 @@ int lzkp_vk_load(const uint8_t *vk_bytes, size_t len, lzkp_vk **out);
 void lzkp_vk_free(lzkp_vk *vk);
 int lzkp_verify_batch(lzkp_vk *vk, size_t n, const uint8_t *proofs, const uint8_t *public_inputs, size_t n_pub,
                       uint8_t *ok_out);
+/* lzkp_verify_batch with proofs, public inputs and ok in device memory of the key's device (the one it was loaded on),
+ * asynchronous on `stream` (cudaStream_t or NULL): same layouts, same forms, same decisions.  Like every *_device entry
+ * point it returns once the work is ENQUEUED, and the caller's buffers must stay valid until `stream` has run it; calls
+ * on one key from several streams, host-buffer calls included, are ordered by the key's last-use event.  The combined
+ * form's coefficients are a ChaCha20 expansion, on the device, of a 256-bit seed read from the OS at every call, and
+ * groups whose combined check fails are re-verified on the device: nothing is copied to or from the host and the call
+ * does not wait for the device, except when the call needs more scratch memory than the key holds - then it first waits
+ * for the key's in-flight calls.
+ *   LZKP_E_INVALID      a NULL buffer (n > 0), proofs or public inputs not 16-byte aligned, or a buffer that is host
+ *                       memory or on another device
+ *   LZKP_E_UNSUPPORTED  `stream` is being captured: the seed is drawn when the work is enqueued, so every replay of a
+ *                       captured graph would reuse the same coefficients and the combined check would lose its soundness
+ * A wrong n_pub enqueues a zeroing of ok (every proof rejected); n == 0 enqueues nothing. */
+int lzkp_verify_batch_device(lzkp_vk *vk, size_t n, const void *d_proofs, const void *d_public_inputs, size_t n_pub,
+                             void *d_ok, void *stream);
 /* info[0..4) = n_pub, bytes of the byte-window tables on the device, latency form available (1/0), combined form with
  * the cooperative check available (1/0) */
 int lzkp_vk_info(const lzkp_vk *vk, uint64_t info[4]);

@@ -57,6 +57,8 @@ extern "C" {
     pub fn lzkp_vk_info(vk: *const lzkp_vk, info: *mut u64) -> c_int;
     pub fn lzkp_verify_batch(vk: *mut lzkp_vk, n: usize, proofs: *const u8, public_inputs: *const u8, n_pub: usize,
                              ok_out: *mut u8) -> c_int;
+    pub fn lzkp_verify_batch_device(vk: *mut lzkp_vk, n: usize, d_proofs: *const c_void, d_public_inputs: *const c_void,
+                                    n_pub: usize, d_ok: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn lzkp_commit_value_snark(value: u64, out: *mut u8) -> c_int;
     pub fn lzkp_msm_g1(bases: *const u8, scalars: *const u8, n: usize, out: *mut u8) -> c_int;
     pub fn lzkp_msm_g2(bases: *const u8, scalars: *const u8, n: usize, out: *mut u8) -> c_int;

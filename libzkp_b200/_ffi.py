@@ -78,6 +78,7 @@ SIGNATURES = {
     "lzkp_vk_free": (None, [_vp]),
     "lzkp_vk_info": (_int, [_vp, C.POINTER(_u64)]),
     "lzkp_verify_batch": (_int, [_vp, _sz, _vp, _vp, _sz, _vp]),
+    "lzkp_verify_batch_device": (_int, [_vp, _sz, _vp, _vp, _sz, _vp, _vp]),
     "lzkp_commit_value_snark": (_int, [_u64, _vp]),
 }
 

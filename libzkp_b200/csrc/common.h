@@ -62,6 +62,17 @@ struct DBuf {
 
 namespace lzkp {
 namespace eng {
+// Buffers shared by calls on several streams: every user makes its stream wait on the buffers' last use (the event is
+// created by the first user) and records it after its own last enqueue.
+inline int event_acquire(cudaEvent_t &last_use, cudaStream_t st) {
+    if (!last_use) CUDA_TRY(cudaEventCreateWithFlags(&last_use, cudaEventDisableTiming));
+    else CUDA_TRY(cudaStreamWaitEvent(st, last_use, 0));
+    return LZKP_OK;
+}
+inline int event_release(cudaEvent_t last_use, cudaStream_t st) {
+    CUDA_TRY(cudaEventRecord(last_use, st));
+    return LZKP_OK;
+}
 template <class T>
 inline int upload(DBuf &b, const std::vector<T> &v) {
     TRY(b.alloc(v.size() * sizeof(T)));

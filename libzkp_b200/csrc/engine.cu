@@ -139,15 +139,8 @@ struct Workspace {
     cudaEvent_t last_use = nullptr;
     ~Workspace() { if (last_use) cudaEventDestroy(last_use); }
 };
-static int ws_acquire(Workspace &ws, cudaStream_t st) {
-    if (!ws.last_use) CUDA_TRY(cudaEventCreateWithFlags(&ws.last_use, cudaEventDisableTiming));
-    else CUDA_TRY(cudaStreamWaitEvent(st, ws.last_use, 0));
-    return LZKP_OK;
-}
-static int ws_release(Workspace &ws, cudaStream_t st) {
-    CUDA_TRY(cudaEventRecord(ws.last_use, st));
-    return LZKP_OK;
-}
+static int ws_acquire(Workspace &ws, cudaStream_t st) { return event_acquire(ws.last_use, st); }
+static int ws_release(Workspace &ws, cudaStream_t st) { return event_release(ws.last_use, st); }
 
 // pk->stream is a BLOCKING stream on purpose: setup-time uploads use synchronous cudaMemcpy from pageable
 // memory, whose DMA tail is only ordered against the legacy default stream and streams that synchronise
@@ -1777,6 +1770,13 @@ int lzkp_verify_batch(lzkp_vk *vk, size_t n, const uint8_t *proofs, const uint8_
     if (!vk || (n && (!proofs || !ok_out || (n_pub && !public_inputs)))) return fail(LZKP_E_INVALID, "null argument");
     TRY(ensure_device());
     return verify_batch(vk->v, n, proofs, public_inputs, n_pub, ok_out);
+}
+int lzkp_verify_batch_device(lzkp_vk *vk, size_t n, const void *d_proofs, const void *d_public_inputs, size_t n_pub,
+                             void *d_ok, void *stream) {
+    if (!vk || (n && (!d_proofs || !d_ok || (n_pub && !d_public_inputs)))) return fail(LZKP_E_INVALID, "null argument");
+    TRY(ensure_device());
+    return verify_batch_device(vk->v, n, (const uint8_t *)d_proofs, (const uint8_t *)d_public_inputs, n_pub, (uint8_t *)d_ok,
+                               (cudaStream_t)stream);
 }
 
 int lzkp_commit_value_snark(uint64_t value, uint8_t out[32]) {

@@ -13,11 +13,14 @@
 //   * one proof per lane (k_verify4): keys without the latency form's tables, no OS entropy, large failing ranges.
 // Keys above kCoopScanMax public inputs take the same forms; there vk_x of each proof comes from its own kernel (k_vkx)
 // and the combined form's scalar sums from k_rlc_input_sums.
+// lzkp_verify_batch_device runs the same stages on the caller's stream from device buffers; its coefficients come from
+// k_rlc_rho and its failing groups are listed by k_rlc_failed and re-verified by the Listed instantiations of the forms.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <vector>
 
+#include "chacha20.cuh"
 #include "dev_util.cuh"
 #include "host_util.h"
 #include "coop.cuh"
@@ -106,15 +109,29 @@ __global__ void k_vk_prepare(VkDev *vk) {
 //   warp 1: vk_x, Miller(vk_x, -gamma)                   warp 3: B in the r-torsion subgroup?
 // vkx (keys above kCoopScanMax inputs that have the byte-window tables): vk_x of every proof, computed by k_vkx; warp 1
 // then only checks that the inputs are canonical.
+// Listed: the proofs of the list k_rlc_failed wrote (lzkp_verify_batch_device re-verifying failing groups without the
+// host).  Entry i of the launch is proof list[i]; the kernel runs only while i < F = *count and lo < F <= hi, the
+// range of F for which the host path would pick this form, so that one launch per form covers every F.
+struct ListGate {
+    const uint32_t *list, *count;
+    uint32_t lo, hi;
+};
+template <bool Listed>
 __global__ void __launch_bounds__(128) k_verify4(const VkDev *__restrict__ vk, const G1Affine *__restrict__ gamma_abc,
                                                  uint32_t n_pub, const uint8_t *__restrict__ proofs,
                                                  const Fr *__restrict__ inputs, const G1Affine *__restrict__ vkx, uint32_t n,
-                                                 uint8_t *__restrict__ ok) {
+                                                 uint8_t *__restrict__ ok, ListGate lg) {
     extern __shared__ uint4 smem_raw[];
     Fq12 *sf = reinterpret_cast<Fq12 *>(smem_raw);                       // [2][32] Miller values of warps 1, 2
     __shared__ uint8_t sgood[4][32];
-    const uint32_t role = threadIdx.x >> 5, lane = threadIdx.x & 31, p = blockIdx.x * 32 + lane;
+    const uint32_t role = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint32_t p = blockIdx.x * 32 + lane;
+    if (Listed) {
+        n = *lg.count;
+        if (n <= lg.lo || n > lg.hi) return;
+    }
     const bool live = p < n;
+    if (Listed && live) p = lg.list[p];
     const uint8_t *pb = proofs + (size_t)p * 256;
     Fq12 f;
     bool good = true;
@@ -538,15 +555,22 @@ __device__ __forceinline__ void set_emb(FChain &c, const G1Affine &P) {
 enum CoopRole { kAbUpper = 0, kLines = 1, kAbLower = 2, kLadder = 3, kGamma = 4, kIdle = 5, kDelta = 6 };
 // MIN_CTAS = 1: all the registers the code wants (250; one CTA per SM) for calls of at most one proof per SM; MIN_CTAS = 2: 128
 // registers, two proofs per SM side by side - 10 % slower each (1.99 against 1.80 ms), 1.5x the throughput from 149 proofs on.
-template <int MIN_CTAS>
+// Listed: as for k_verify4, CTA i verifies proof list[i] while i < F and lo < F <= hi.
+template <int MIN_CTAS, bool Listed>
 __global__ void __launch_bounds__(kCoopThreads, MIN_CTAS) k_verify_coop(const VkDev *__restrict__ vk, const G1Affine *__restrict__ gamma_abc,
                                                               const G1Affine *__restrict__ tab, const Fq2 *__restrict__ lines_gamma,
                                                               const Fq2 *__restrict__ lines_delta, uint32_t n_pub,
                                                               const uint8_t *__restrict__ proofs, const uint8_t *__restrict__ inputs,
-                                                              const G1Affine *__restrict__ vkx, uint8_t *__restrict__ ok) {
+                                                              const G1Affine *__restrict__ vkx, uint8_t *__restrict__ ok, ListGate lg) {
     extern __shared__ uint4 smem_raw[];
     CoopSmem &sm = *reinterpret_cast<CoopSmem *>(smem_raw);
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31, p = blockIdx.x;
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint32_t p = blockIdx.x;
+    if (Listed) {
+        const uint32_t F = *lg.count;
+        if (p >= F || F <= lg.lo || F > lg.hi) return;
+        p = lg.list[p];
+    }
     const uint8_t *pb = proofs + (size_t)p * 256;
     const uint8_t *x = inputs + (size_t)p * n_pub * 32;
     coop_prologue(sm);
@@ -777,6 +801,54 @@ __global__ void __launch_bounds__(128) k_rlc_inputs2(const Fr *__restrict__ gS, 
     if (lane == 0) st_vec(gX + t, acc);
 }
 
+// ---- the combined form without the host (lzkp_verify_batch_device)
+// rho of every proof from a 256-bit seed, thread = ChaCha20 block of four proofs (chacha20.cuh): the call passes the seed
+// as a kernel argument, so nothing is staged in host memory that a later call could overwrite before the copy ran.
+struct RhoSeed { uint32_t w[8]; };
+__global__ void __launch_bounds__(128) k_rlc_rho(RhoSeed seed, uint32_t n, uint32_t *__restrict__ rho) {
+    const uint32_t blk = blockIdx.x * blockDim.x + threadIdx.x;
+    if (blk >= (n + 3) / 4) return;
+    rlc_rho_block(seed.w, blk, n, rho);
+}
+// list[0 .. F) = the proofs of every group whose combined check failed, ascending, and count[0] = F.  One CTA: a scan of
+// the group flags in chunks of one flag per thread (1024 groups at 65 536 proofs).
+constexpr uint32_t kFailedThreads = 1024;
+__global__ void __launch_bounds__(kFailedThreads) k_rlc_failed(const uint8_t *__restrict__ group_ok, uint32_t n, uint32_t groups,
+                                                               uint32_t *__restrict__ list, uint32_t *__restrict__ count) {
+    __shared__ uint32_t s_warp[kFailedThreads / 32], s_base;
+    const uint32_t t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    if (t == 0) s_base = 0;
+#pragma unroll 1
+    for (uint32_t g0 = 0; g0 < groups; g0 += kFailedThreads) {
+        const uint32_t g = g0 + t, lo = g * kRlcGroup;
+        const uint32_t cnt = g < groups && !group_ok[g] ? min(n - lo, kRlcGroup) : 0;
+        uint32_t incl = cnt;                                              // inclusive scan: warp, then across warps
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            const uint32_t v = __shfl_up_sync(0xffffffffu, incl, off);
+            if (lane >= (uint32_t)off) incl += v;
+        }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        if (warp == 0) {
+            uint32_t w = s_warp[lane];
+#pragma unroll
+            for (int off = 1; off < 32; off <<= 1) {
+                const uint32_t v = __shfl_up_sync(0xffffffffu, w, off);
+                if (lane >= (uint32_t)off) w += v;
+            }
+            s_warp[lane] = w;
+        }
+        __syncthreads();
+        const uint32_t base = s_base + (warp ? s_warp[warp - 1] : 0) + incl - cnt;
+        for (uint32_t k = 0; k < cnt; k++) list[base + k] = lo + k;
+        __syncthreads();
+        if (t == 0) s_base += s_warp[kFailedThreads / 32 - 1];
+        __syncthreads();
+    }
+    if (t == 0) *count = s_base;
+}
+
 // ---- vk_x of every proof of a call, keys above kCoopScanMax public inputs.  The latency form's GAMMA warp scans all
 // n_pub x 32 (input, byte) pairs itself (coop::vkx_from_tables), and the Miller loop against -gamma waits for it: at 2049
 // inputs that is ~2000 steps on the critical path.  Here one CTA per proof: warp w takes the slices w, w + warps, ... of
@@ -788,11 +860,18 @@ constexpr uint32_t kVkxWarps = 8;
 // Inputs per slice.  At 2049 inputs (B200, 1000 W) k_vkx takes 0.22 / 0.49 / 1.07 ms for 1 / 64 / 444 proofs with slices of 64;
 // 32 and 128 tie at 1 and 64 proofs and lose at 444 (1.16, 1.18 ms), 256 and 512 lose at 64 proofs (0.57, 0.83 ms).
 constexpr uint32_t kVkxSlice = 64;
+// Listed: CTA i computes vk_x of proof list[i] while i < F (every F: all re-verifying forms read it).
+template <bool Listed>
 __global__ void __launch_bounds__(kVkxWarps * 32) k_vkx(const G1Affine *__restrict__ tab, const G1Affine *__restrict__ gamma_abc,
                                                         uint32_t n_pub, uint32_t slice, const uint8_t *__restrict__ inputs,
-                                                        G1Affine *__restrict__ vkx) {
+                                                        G1Affine *__restrict__ vkx, ListGate lg) {
     __shared__ G1XYZZ part[kVkxWarps * 32];
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31, warps = blockDim.x >> 5, p = blockIdx.x;
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31, warps = blockDim.x >> 5;
+    uint32_t p = blockIdx.x;
+    if (Listed) {
+        if (p >= *lg.count) return;
+        p = lg.list[p];
+    }
     const uint4 *x = reinterpret_cast<const uint4 *>(inputs + (size_t)p * n_pub * 32);
     G1XYZZ acc = G1XYZZ::inf();
     if (threadIdx.x == 0) acc = G1XYZZ::from_affine(ldg_vec(gamma_abc));
@@ -938,14 +1017,36 @@ namespace eng {
 
 struct VerifyingKeyDev {
     DBuf vk, gamma_abc;
-    DBuf d_p, d_x, d_ok;          // grow-only staging of a batch (calls on one key serialize on mu)
+    DBuf d_p, d_x, d_ok;          // grow-only staging of lzkp_verify_batch's host buffers
     DBuf d_rho, d_f, d_rc, d_sx, d_gF, d_gC, d_gS, d_gX, d_gok;     // random-linear-combination path (large batches)
+    DBuf d_list;                                                                 // failing groups' proofs and their count (k_rlc_failed)
     DBuf lines_gamma, lines_delta, lines_beta, tab;                             // latency form (coop.cuh): prepared lines, vk_x byte-window tables
     DBuf d_vkx;                                                                  // vk_x per proof (k_vkx; keys above kCoopScanMax inputs)
     bool coop_ok = false;
     uint32_t n_pub = 0;
+    int device = 0;                                                              // the device the key was loaded on
+    // Last use of the per-call buffers above, on whatever stream it was enqueued (lzkp_verify_batch_device returns before
+    // its work has run).  Every call waits on it in its stream before touching them and records it after its last
+    // enqueue: event_acquire / event_release.  mu only orders the ENQUEUES.
+    cudaEvent_t last_use = nullptr;
     std::mutex mu;
+    ~VerifyingKeyDev() {
+        if (last_use) { cudaEventSynchronize(last_use); cudaEventDestroy(last_use); }
+    }
 };
+// A call that needs a larger buffer than the key holds first waits on the host for the calls still using the old one.
+static int grow(VerifyingKeyDev *V, DBuf &b, size_t bytes) {
+    if (bytes <= b.bytes) return LZKP_OK;
+    if (V->last_use) CUDA_TRY(cudaEventSynchronize(V->last_use));
+    return b.alloc(bytes);
+}
+// size x count bytes from the OS CSPRNG (the soundness of the combined check rests on their unpredictability)
+static bool os_entropy(void *dst, size_t size, size_t count) {
+    FILE *ur = fopen("/dev/urandom", "rb");
+    const bool got = ur && fread(dst, size, count, ur) == count;
+    if (ur) fclose(ur);
+    return got;
+}
 
 // The latency and combined forms' per-key data: prepared lines of -gamma / -delta / beta and the byte-window tables of
 // gamma_abc and alpha, (n_pub + 2) x 32 x 255 affine points = 0.52 MB per public input (68.4 MB for the 129 inputs of the
@@ -1040,6 +1141,7 @@ int vk_load(const uint8_t *bytes, size_t len, VerifyingKeyDev **out) {
     VerifyingKeyDev *V = new (std::nothrow) VerifyingKeyDev();
     if (!V) return fail(LZKP_E_NOMEM, "host allocation failed");
     V->n_pub = (uint32_t)cnt - 1;
+    V->device = current_device();
     struct Packed { host::G1Canon alpha; host::G2Canon beta, gneg, dneg; } pk{alpha, beta, neg2(gamma), neg2(delta)};
     static_assert(sizeof(Packed) == sizeof(G1Affine) + 3 * sizeof(G2Affine), "layout");
     int rc = V->vk.alloc(sizeof(VkDev));
@@ -1067,17 +1169,15 @@ void vk_info(const VerifyingKeyDev *V, uint64_t info[4]) {
     info[3] = V->coop_ok ? 1 : 0;          // the combined form with the cooperative check from 3 x SMs + 1 proofs
 }
 
-int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint8_t *inputs, size_t n_pub, uint8_t *ok_out) {
-    std::lock_guard<std::mutex> lk(V->mu);
-    if (n_pub != V->n_pub) {                   // wrong number of public inputs: nothing verifies (reference: Err -> false)
-        memset(ok_out, 0, n);
-        return LZKP_OK;
-    }
-    if (n == 0) return LZKP_OK;
-    DBuf &d_p = V->d_p, &d_x = V->d_x, &d_ok = V->d_ok;
-    TRY(d_p.ensure(n * 256)); TRY(d_x.ensure(n * std::max<size_t>(n_pub, 1) * 32)); TRY(d_ok.ensure(n));
-    CUDA_TRY(cudaMemcpy(d_p.p, proofs, n * 256, cudaMemcpyHostToDevice));
-    if (n_pub) CUDA_TRY(cudaMemcpy(d_x.p, inputs, n * n_pub * 32, cudaMemcpyHostToDevice));
+// Picks the form for n proofs and enqueues its stages on `st`, from proofs / inputs / ok in device memory.  The one
+// stage sequence of both entry points; on_device selects the two places where they differ:
+//   * the combined form's coefficients: 16 B per proof read from the OS and uploaded (lzkp_verify_batch), or a 256-bit
+//     seed read from the OS and expanded on the device by k_rlc_rho (lzkp_verify_batch_device);
+//   * groups whose combined check failed: their flags read back and their ranges re-verified from the host, or listed
+//     by k_rlc_failed and re-verified by one gated launch per form (no host round trip).
+// The caller holds V->mu and has made `st` wait on V->last_use.
+static int enqueue_verify(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint8_t *inputs, size_t n_pub, uint8_t *ok,
+                          cudaStream_t st, bool on_device) {
     // Calls of up to coop_max proofs are bound by ONE proof's dependent chain: there a proof gets a whole CTA whose warps
     // and lanes share the pairing's arithmetic (coop.cuh): 1 / 64 / 148 proofs in 1.8 / 1.9 / 2.2 ms with one CTA per SM,
     // 296 / 444 proofs in 2.7 / 5.2 ms with two per SM, against 5.9 ms for the random-linear-combination form at any
@@ -1087,28 +1187,30 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
     const size_t coop_max = getenv("LZKP_VERIFY_COOP_MAX") ? (size_t)atoll(getenv("LZKP_VERIFY_COOP_MAX")) : (size_t)3 * sm_count;
     // Keys above kCoopScanMax inputs: vk_x of the proofs of a range comes from k_vkx, for the latency form and k_verify4 alike.
     const bool vkx_kernel = V->coop_ok && n_pub > kCoopScanMax;
-    if (vkx_kernel) TRY(V->d_vkx.ensure(n * sizeof(G1Affine)));
+    if (vkx_kernel) TRY(grow(V, V->d_vkx, n * sizeof(G1Affine)));
+    const uint32_t vkx_warps = std::min<uint32_t>(kVkxWarps, ((uint32_t)n_pub + kVkxSlice - 1) / kVkxSlice);
+    const ListGate unlisted{nullptr, nullptr, 0, 0};
     auto verify_range = [&](size_t off, size_t cnt) {             // independent verification of proofs [off, off + cnt)
         const G1Affine *vkx = nullptr;
         if (vkx_kernel) {
-            const uint32_t warps = std::min<uint32_t>(kVkxWarps, ((uint32_t)n_pub + kVkxSlice - 1) / kVkxSlice);
-            LAUNCH(k_vkx, (unsigned)cnt, warps * 32, 0, 0, V->tab.as<G1Affine>(), V->gamma_abc.as<G1Affine>(), (uint32_t)n_pub, kVkxSlice,
-                   d_x.as<uint8_t>() + off * n_pub * 32, V->d_vkx.as<G1Affine>() + off);
+            LAUNCH(k_vkx<false>, (unsigned)cnt, vkx_warps * 32, 0, st, V->tab.as<G1Affine>(), V->gamma_abc.as<G1Affine>(), (uint32_t)n_pub,
+                   kVkxSlice, inputs + off * n_pub * 32, V->d_vkx.as<G1Affine>() + off, unlisted);
             vkx = V->d_vkx.as<G1Affine>() + off;
         }
         if (V->coop_ok && cnt <= coop_max) {
             if (cnt <= (size_t)sm_count)
-                LAUNCH(k_verify_coop<1>, (unsigned)cnt, kCoopThreads, sizeof(CoopSmem), 0, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
+                LAUNCH((k_verify_coop<1, false>), (unsigned)cnt, kCoopThreads, sizeof(CoopSmem), st, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
                        V->tab.as<G1Affine>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(), (uint32_t)n_pub,
-                       d_p.as<uint8_t>() + off * 256, d_x.as<uint8_t>() + off * n_pub * 32, vkx, d_ok.as<uint8_t>() + off);
+                       proofs + off * 256, inputs + off * n_pub * 32, vkx, ok + off, unlisted);
             else
-                LAUNCH(k_verify_coop<2>, (unsigned)cnt, kCoopThreads, sizeof(CoopSmem), 0, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
+                LAUNCH((k_verify_coop<2, false>), (unsigned)cnt, kCoopThreads, sizeof(CoopSmem), st, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
                        V->tab.as<G1Affine>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(), (uint32_t)n_pub,
-                       d_p.as<uint8_t>() + off * 256, d_x.as<uint8_t>() + off * n_pub * 32, vkx, d_ok.as<uint8_t>() + off);
+                       proofs + off * 256, inputs + off * n_pub * 32, vkx, ok + off, unlisted);
             return;
         }
-        LAUNCH(k_verify4, (unsigned)((cnt + 31) / 32), 128, 64 * sizeof(Fq12), 0, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
-               (uint32_t)n_pub, d_p.as<uint8_t>() + off * 256, d_x.as<Fr>() + off * n_pub, vkx, (uint32_t)cnt, d_ok.as<uint8_t>() + off);
+        LAUNCH(k_verify4<false>, (unsigned)((cnt + 31) / 32), 128, 64 * sizeof(Fq12), st, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
+               (uint32_t)n_pub, proofs + off * 256, reinterpret_cast<const Fr *>(inputs) + off * n_pub, vkx, (uint32_t)cnt, ok + off,
+               unlisted);
     };
     // Above the latency form's range the random-linear-combination form takes over: 2.4x less work per proof (one Miller
     // loop instead of three, one final exponentiation per 64 proofs) and, with the cooperative combined check, a short
@@ -1119,42 +1221,40 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
     if (n < rlc_min || n > 0xFFFFFFFFull) {
         static const bool timing = getenv("LZKP_VERIFY_TIMING") != nullptr;
         cudaEvent_t e0 = nullptr, e1 = nullptr;
-        if (timing) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, 0); }
+        const bool timed = timing && !on_device;
+        if (timed) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, st); }
         verify_range(0, n);
-        if (timing) {
-            cudaEventRecord(e1, 0); cudaEventSynchronize(e1);
+        if (timed) {
+            cudaEventRecord(e1, st); cudaEventSynchronize(e1);
             float ms = 0; cudaEventElapsedTime(&ms, e0, e1);
             fprintf(stderr, "lzkp verify_batch: %zu proofs, kernel %.3f ms (events)\n", n, ms);
             cudaEventDestroy(e0); cudaEventDestroy(e1);
         }
-        CUDA_TRY(cudaMemcpy(ok_out, d_ok.p, n, cudaMemcpyDeviceToHost));
-        CUDA_TRY(cudaGetLastError());
         return LZKP_OK;
     }
     const uint32_t ctas = (uint32_t)((n + 31) / 32), groups = (uint32_t)((n + kRlcGroup - 1) / kRlcGroup), np1 = (uint32_t)n_pub + 1;
-    std::vector<uint32_t> rho(n * 4);
-    {   // 128-bit coefficients from the OS CSPRNG (the soundness of the combined check rests on their unpredictability)
-        FILE *ur = fopen("/dev/urandom", "rb");
-        const bool got = ur && fread(rho.data(), 16, n, ur) == n;
-        if (ur) fclose(ur);
-        if (!got) {                                                // no entropy source: verify independently instead
-            verify_range(0, n);
-            CUDA_TRY(cudaMemcpy(ok_out, d_ok.p, n, cudaMemcpyDeviceToHost));
-            CUDA_TRY(cudaGetLastError());
-            return LZKP_OK;
-        }
+    std::vector<uint32_t> rho(on_device ? 0 : n * 4);
+    RhoSeed seed;
+    if (!(on_device ? os_entropy(seed.w, sizeof(seed.w), 1) : os_entropy(rho.data(), 16, n))) {
+        verify_range(0, n);                                       // no entropy source: verify independently instead
+        return LZKP_OK;
     }
-    TRY(V->d_rho.ensure(n * 16)); TRY(V->d_f.ensure(n * sizeof(Fq12))); TRY(V->d_rc.ensure(n * sizeof(G1XYZZ)));
+    TRY(grow(V, V->d_rho, n * 16)); TRY(grow(V, V->d_f, n * sizeof(Fq12))); TRY(grow(V, V->d_rc, n * sizeof(G1XYZZ)));
     static const bool tail_lanes = getenv("LZKP_RLC_TAIL_LANES") != nullptr;      // A/B switch: the lane-per-group tail
     // Keys above kCoopScanMax inputs: the scalar sums per (group, input) in k_rlc_input_sums, not in the per-proof kernel.  At
     // 2049 inputs (B200, 1000 W) the per-proof kernel's sums strand outlasts its Miller loop: k_rlc_prepare 5.83 against
     // 3.97 ms at 445 proofs, 6.89 against 4.12 at 4096; k_rlc_input_sums itself takes 0.04 / 0.18 ms.
     const bool input_sums = V->coop_ok && !tail_lanes && n_pub > kCoopScanMax;
-    if (!input_sums) TRY(V->d_sx.ensure((size_t)ctas * np1 * sizeof(Fr)));
-    TRY(V->d_gF.ensure((size_t)groups * sizeof(Fq12))); TRY(V->d_gC.ensure((size_t)groups * sizeof(G1XYZZ)));
-    TRY(V->d_gS.ensure((size_t)groups * np1 * sizeof(Fr))); TRY(V->d_gX.ensure((size_t)groups * (np1 + 1) * sizeof(G1XYZZ)));
-    TRY(V->d_gok.ensure(groups));
-    CUDA_TRY(cudaMemcpy(V->d_rho.p, rho.data(), n * 16, cudaMemcpyHostToDevice));
+    if (!input_sums) TRY(grow(V, V->d_sx, (size_t)ctas * np1 * sizeof(Fr)));
+    TRY(grow(V, V->d_gF, (size_t)groups * sizeof(Fq12))); TRY(grow(V, V->d_gC, (size_t)groups * sizeof(G1XYZZ)));
+    TRY(grow(V, V->d_gS, (size_t)groups * np1 * sizeof(Fr))); TRY(grow(V, V->d_gX, (size_t)groups * (np1 + 1) * sizeof(G1XYZZ)));
+    TRY(grow(V, V->d_gok, groups));
+    if (on_device) {
+        TRY(grow(V, V->d_list, (n + 1) * sizeof(uint32_t)));
+        LAUNCH(k_rlc_rho, (unsigned)(((n + 3) / 4 + 127) / 128), 128, 0, st, seed, (uint32_t)n, V->d_rho.as<uint32_t>());
+    } else {
+        CUDA_TRY(cudaMemcpy(V->d_rho.p, rho.data(), n * 16, cudaMemcpyHostToDevice));
+    }
     // One launch per stage for the whole batch.  (Measured: cutting the batch into 16 384-proof chunks so that a chunk's
     // tail runs under the next chunk's k_rlc_prepare on a second stream is SLOWER - 98 to 108 ms against 81 ms at 65 536
     // proofs: the per-proof kernel is a latency-bound chain per CTA, and four 512-CTA launches fill whole waves worse
@@ -1167,35 +1267,61 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
     // 13.3 - 13.7 ms for the sequential kernel at 12 288 - 18 944 proofs - rejected)
     const bool prep_roles = force ? atoi(force) != 0 : n <= (size_t)sm_count * 2 * 32;
     Fr *sx = input_sums ? nullptr : V->d_sx.as<Fr>();
+    const Fr *x = reinterpret_cast<const Fr *>(inputs);
     if (prep_roles)
-        LAUNCH(k_rlc_prepare, ctas, 128, 32 * (sizeof(Fq12) + sizeof(G1Affine)), 0, V->vk.as<VkDev>(), (uint32_t)n_pub, d_p.as<uint8_t>(), d_x.as<Fr>(), V->d_rho.as<uint32_t>(),
-               (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), sx, d_ok.as<uint8_t>());
+        LAUNCH(k_rlc_prepare, ctas, 128, 32 * (sizeof(Fq12) + sizeof(G1Affine)), st, V->vk.as<VkDev>(), (uint32_t)n_pub, proofs, x, V->d_rho.as<uint32_t>(),
+               (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), sx, ok);
     else
-        LAUNCH(k_rlc_prepare_seq, (ctas + 1) / 2, 64, 0, 0, V->vk.as<VkDev>(), (uint32_t)n_pub, d_p.as<uint8_t>(), d_x.as<Fr>(),
-               V->d_rho.as<uint32_t>(), (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), sx, d_ok.as<uint8_t>());
+        LAUNCH(k_rlc_prepare_seq, (ctas + 1) / 2, 64, 0, st, V->vk.as<VkDev>(), (uint32_t)n_pub, proofs, x,
+               V->d_rho.as<uint32_t>(), (uint32_t)n, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), sx, ok);
     if (V->coop_ok && !tail_lanes) {
         if (input_sums)
-            LAUNCH(k_rlc_input_sums, dim3(groups, (np1 + 127) / 128), 128, 0, 0, d_x.as<Fr>(), V->d_rho.as<uint32_t>(), d_ok.as<uint8_t>(),
+            LAUNCH(k_rlc_input_sums, dim3(groups, (np1 + 127) / 128), 128, 0, st, x, V->d_rho.as<uint32_t>(), ok,
                    (uint32_t)n, (uint32_t)n_pub, V->d_gS.as<Fr>());
         else
-            LAUNCH(k_rlc_scalars, (groups * np1 + 127) / 128, 128, 0, 0, V->d_sx.as<Fr>(), (uint32_t)n, (uint32_t)n_pub, groups, V->d_gS.as<Fr>());
-        LAUNCH(k_rlc_inputs2, (groups * (np1 + 1) + 3) / 4, 128, 0, 0, V->d_gS.as<Fr>(), V->tab.as<G1Affine>(), (uint32_t)n_pub, groups,
+            LAUNCH(k_rlc_scalars, (groups * np1 + 127) / 128, 128, 0, st, V->d_sx.as<Fr>(), (uint32_t)n, (uint32_t)n_pub, groups, V->d_gS.as<Fr>());
+        LAUNCH(k_rlc_inputs2, (groups * (np1 + 1) + 3) / 4, 128, 0, st, V->d_gS.as<Fr>(), V->tab.as<G1Affine>(), (uint32_t)n_pub, groups,
                V->d_gX.as<G1XYZZ>());
         if (groups <= 2u * (uint32_t)sm_count)
-            LAUNCH(k_rlc_tail_coop<2>, groups, 128, sizeof(TailSmem), 0, V->vk.as<VkDev>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(),
+            LAUNCH(k_rlc_tail_coop<2>, groups, 128, sizeof(TailSmem), st, V->vk.as<VkDev>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(),
                    V->lines_beta.as<Fq2>(), V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), V->d_gX.as<G1XYZZ>(), (uint32_t)n, (uint32_t)n_pub,
                    V->d_gok.as<uint8_t>());
         else
-            LAUNCH(k_rlc_tail_coop<4>, groups, 128, sizeof(TailSmem), 0, V->vk.as<VkDev>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(),
+            LAUNCH(k_rlc_tail_coop<4>, groups, 128, sizeof(TailSmem), st, V->vk.as<VkDev>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(),
                    V->lines_beta.as<Fq2>(), V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), V->d_gX.as<G1XYZZ>(), (uint32_t)n, (uint32_t)n_pub,
                    V->d_gok.as<uint8_t>());
     } else {
-    LAUNCH(k_rlc_reduce, (groups + 63) / 64, 64, 0, 0, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), V->d_sx.as<Fr>(), (uint32_t)n,
+    LAUNCH(k_rlc_reduce, (groups + 63) / 64, 64, 0, st, V->d_f.as<Fq12>(), V->d_rc.as<G1XYZZ>(), V->d_sx.as<Fr>(), (uint32_t)n,
            (uint32_t)n_pub, groups, V->d_gF.as<Fq12>(), V->d_gC.as<G1XYZZ>(), V->d_gS.as<Fr>());
-    LAUNCH(k_rlc_inputs, (groups * np1 + 63) / 64, 64, 0, 0, V->d_gS.as<Fr>(), V->gamma_abc.as<G1Affine>(), (uint32_t)n_pub, groups,
+    LAUNCH(k_rlc_inputs, (groups * np1 + 63) / 64, 64, 0, st, V->d_gS.as<Fr>(), V->gamma_abc.as<G1Affine>(), (uint32_t)n_pub, groups,
            V->d_gX.as<G1XYZZ>());
-    LAUNCH(k_rlc_tail, (groups + 31) / 32, 128, 96 * sizeof(Fq12), 0, V->vk.as<VkDev>(), V->d_gF.as<Fq12>(), V->d_gC.as<G1XYZZ>(),
+    LAUNCH(k_rlc_tail, (groups + 31) / 32, 128, 96 * sizeof(Fq12), st, V->vk.as<VkDev>(), V->d_gF.as<Fq12>(), V->d_gC.as<G1XYZZ>(),
            V->d_gS.as<Fr>(), V->d_gX.as<G1XYZZ>(), (uint32_t)n_pub, groups, V->d_gok.as<uint8_t>());
+    }
+    if (on_device) {
+        // The failing groups' proofs, listed on the device, are re-verified by the form the host path would pick for
+        // their count F: one launch per form sized for its largest F, whose CTAs leave unless F is in that form's range.
+        uint32_t *list = V->d_list.as<uint32_t>(), *count = list + n;
+        LAUNCH(k_rlc_failed, 1, kFailedThreads, 0, st, V->d_gok.as<uint8_t>(), (uint32_t)n, groups, list, count);
+        const G1Affine *vkx = nullptr;
+        if (vkx_kernel) {
+            LAUNCH(k_vkx<true>, (unsigned)n, vkx_warps * 32, 0, st, V->tab.as<G1Affine>(), V->gamma_abc.as<G1Affine>(), (uint32_t)n_pub,
+                   kVkxSlice, inputs, V->d_vkx.as<G1Affine>(), ListGate{list, count, 0, 0xFFFFFFFFu});
+            vkx = V->d_vkx.as<G1Affine>();
+        }
+        const uint32_t cmax = V->coop_ok ? (uint32_t)std::min<size_t>(coop_max, n) : 0, one = std::min<uint32_t>(cmax, sm_count);
+        if (one)
+            LAUNCH((k_verify_coop<1, true>), one, kCoopThreads, sizeof(CoopSmem), st, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
+                   V->tab.as<G1Affine>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(), (uint32_t)n_pub, proofs, inputs, vkx, ok,
+                   ListGate{list, count, 0, one});
+        if (cmax > (uint32_t)sm_count)
+            LAUNCH((k_verify_coop<2, true>), cmax, kCoopThreads, sizeof(CoopSmem), st, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
+                   V->tab.as<G1Affine>(), V->lines_gamma.as<Fq2>(), V->lines_delta.as<Fq2>(), (uint32_t)n_pub, proofs, inputs, vkx, ok,
+                   ListGate{list, count, (uint32_t)sm_count, cmax});
+        if (n > cmax)
+            LAUNCH(k_verify4<true>, (unsigned)((n + 31) / 32), 128, 64 * sizeof(Fq12), st, V->vk.as<VkDev>(), V->gamma_abc.as<G1Affine>(),
+                   (uint32_t)n_pub, proofs, x, vkx, (uint32_t)n, ok, ListGate{list, count, cmax, 0xFFFFFFFFu});
+        return LZKP_OK;
     }
     std::vector<uint8_t> gok(groups);
     CUDA_TRY(cudaMemcpy(gok.data(), V->d_gok.p, groups, cudaMemcpyDeviceToHost));
@@ -1209,7 +1335,67 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
         verify_range(off, end - off);
         g = h;
     }
+    return LZKP_OK;
+}
+
+// Waits on the key's last use in `st`, enqueues the call and records the last use, even when the enqueue failed halfway.
+static int enqueue_ordered(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint8_t *inputs, size_t n_pub, uint8_t *ok,
+                           cudaStream_t st, bool on_device) {
+    TRY(event_acquire(V->last_use, st));
+    const int rc = enqueue_verify(V, n, proofs, inputs, n_pub, ok, st, on_device);
+    TRY(event_release(V->last_use, st));
+    return rc;
+}
+
+int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint8_t *inputs, size_t n_pub, uint8_t *ok_out) {
+    std::lock_guard<std::mutex> lk(V->mu);
+    if (n_pub != V->n_pub) {                   // wrong number of public inputs: nothing verifies (reference: Err -> false)
+        memset(ok_out, 0, n);
+        return LZKP_OK;
+    }
+    if (n == 0) return LZKP_OK;
+    DBuf &d_p = V->d_p, &d_x = V->d_x, &d_ok = V->d_ok;
+    TRY(grow(V, d_p, n * 256)); TRY(grow(V, d_x, n * std::max<size_t>(n_pub, 1) * 32)); TRY(grow(V, d_ok, n));
+    CUDA_TRY(cudaMemcpy(d_p.p, proofs, n * 256, cudaMemcpyHostToDevice));
+    if (n_pub) CUDA_TRY(cudaMemcpy(d_x.p, inputs, n * n_pub * 32, cudaMemcpyHostToDevice));
+    TRY(enqueue_ordered(V, n, d_p.as<uint8_t>(), d_x.as<uint8_t>(), n_pub, d_ok.as<uint8_t>(), 0, false));
     CUDA_TRY(cudaMemcpy(ok_out, d_ok.p, n, cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaGetLastError());
+    return LZKP_OK;
+}
+
+// Device memory of the key's device, not host memory (cudaPointerGetAttributes: unregistered or pinned host memory).
+static int check_device_buffer(const VerifyingKeyDev *V, const void *p, const char *what) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(LZKP_E_INVALID, std::string(what) + ": not a CUDA pointer");
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != V->device)
+        return fail(LZKP_E_INVALID, std::string(what) + ": not device memory of the key's device");
+    return LZKP_OK;
+}
+
+int verify_batch_device(VerifyingKeyDev *V, size_t n, const uint8_t *d_proofs, const uint8_t *d_inputs, size_t n_pub, uint8_t *d_ok,
+                        cudaStream_t st) {
+    // A graph replay would reuse the coefficients drawn at capture: refuse capture rather than weaken the combined check.
+    cudaStreamCaptureStatus capturing = cudaStreamCaptureStatusNone;
+    CUDA_TRY(cudaStreamIsCapturing(st, &capturing));
+    if (capturing != cudaStreamCaptureStatusNone)
+        return fail(LZKP_E_UNSUPPORTED, "lzkp_verify_batch_device: stream capture is not supported (coefficients are drawn per call)");
+    if (n == 0) return LZKP_OK;
+    // the kernels read proofs and inputs with 128-bit loads
+    if ((reinterpret_cast<uintptr_t>(d_proofs) | reinterpret_cast<uintptr_t>(d_inputs)) & 15)
+        return fail(LZKP_E_INVALID, "lzkp_verify_batch_device: proofs and public inputs must be 16-byte aligned");
+    TRY(check_device_buffer(V, d_proofs, "proofs"));
+    if (n_pub) TRY(check_device_buffer(V, d_inputs, "public inputs"));
+    TRY(check_device_buffer(V, d_ok, "ok"));
+    if (n_pub != V->n_pub) {                   // wrong number of public inputs: nothing verifies
+        CUDA_TRY(cudaMemsetAsync(d_ok, 0, n, st));
+        return LZKP_OK;
+    }
+    std::lock_guard<std::mutex> lk(V->mu);
+    TRY(enqueue_ordered(V, n, d_proofs, d_inputs, n_pub, d_ok, st, true));
     CUDA_TRY(cudaGetLastError());
     return LZKP_OK;
 }

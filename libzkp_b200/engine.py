@@ -383,6 +383,11 @@ class VerifyingKey:
         check(lib().lzkp_verify_batch(self._h, n, _p(proofs), _p(x) if x.size else None, n_pub, _p(ok)))
         return ok.astype(bool)
 
+    def verify_batch_device(self, n: int, d_proofs: int, d_inputs: int, n_pub: int, d_ok: int, stream: int = 0) -> None:
+        """lzkp_verify_batch_device: proofs (n x 256 B), public inputs (n x n_pub x 32 B) and ok (n bytes) are device
+        pointers (ints) on the key's device; asynchronous on `stream`.  Refused on a stream that is being captured."""
+        check(lib().lzkp_verify_batch_device(self._h, n, d_proofs, d_inputs, n_pub, d_ok, stream))
+
     def info(self):
         """(n_pub, table bytes, latency form available, combined form available) of the loaded key."""
         v = (C.c_uint64 * 4)()
