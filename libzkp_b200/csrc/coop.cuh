@@ -651,15 +651,10 @@ __device__ __noinline__ bool ladder_madd(LadderState *st) {
     __syncwarp();
     return true;
 }
-// B (on the twist, not infinity) in the r-torsion subgroup?  The ladder computes [x] B (62 doublings, 27 additions with
-// their independent products on different lanes); lane 0 then finishes the test of pairing.cuh g2_subgroup_from_xp.
-__device__ __noinline__ bool g2_in_subgroup(LadderState *st, const G2Affine &B) {
+// One bit of the ladder: acc = 2 acc, then acc += (bx, by) when `add`.  Special points (acc at infinity or of order two,
+// acc == +-B) take the complete serial formulas on lane 0.
+__device__ __forceinline__ void ladder_step(LadderState *st, bool add) {
     const int lane = lane_id();
-    if (lane == 0) {
-        stq(&st->X, B.x); stq(&st->Y, B.y); stq(&st->ZZ, Fq2::one()); stq(&st->ZZZ, Fq2::one());
-        stq(&st->bx, B.x); stq(&st->by, B.y);
-    }
-    __syncwarp();
     auto serial = [&](bool add) {          // special points: the complete formulas on one lane
         if (lane == 0) {
             G2XYZZ a{ldq(&st->X), ldq(&st->Y), ldq(&st->ZZ), ldq(&st->ZZZ)};
@@ -674,14 +669,23 @@ __device__ __noinline__ bool g2_in_subgroup(LadderState *st, const G2Affine &B) 
         if (lane == 0) sp = ldq(&st->ZZ).is_zero() || ldq(&st->Y).is_zero();
         return __shfl_sync(0xffffffffu, (int)sp, 0) != 0;
     };
-#pragma unroll 1
-    for (int i = 61; i >= 0; i--) {        // bit 62 is the leading one of x
-        if (is_special()) serial(false);
-        else ladder_dbl(st);
-        if ((kBnX >> i) & 1ull) {
-            if (is_special() || !ladder_madd(st)) serial(true);
-        }
+    if (is_special()) serial(false);
+    else ladder_dbl(st);
+    if (add) {
+        if (is_special() || !ladder_madd(st)) serial(true);
     }
+}
+// B (on the twist, not infinity) in the r-torsion subgroup?  The ladder computes [x] B (62 doublings, 27 additions with
+// their independent products on different lanes); lane 0 then finishes the test of pairing.cuh g2_subgroup_from_xp.
+__device__ __noinline__ bool g2_in_subgroup(LadderState *st, const G2Affine &B) {
+    const int lane = lane_id();
+    if (lane == 0) {
+        stq(&st->X, B.x); stq(&st->Y, B.y); stq(&st->ZZ, Fq2::one()); stq(&st->ZZZ, Fq2::one());
+        stq(&st->bx, B.x); stq(&st->by, B.y);
+    }
+    __syncwarp();
+#pragma unroll 1
+    for (int i = 61; i >= 0; i--) ladder_step(st, ((kBnX >> i) & 1ull) != 0);     // bit 62 is the leading one of x
     bool ok = false;
     if (lane == 0) ok = g2_subgroup_from_xp(B, G2XYZZ{ldq(&st->X), ldq(&st->Y), ldq(&st->ZZ), ldq(&st->ZZZ)});
     return __shfl_sync(0xffffffffu, (int)ok, 0) != 0;

@@ -38,25 +38,30 @@ def f2sqrt(a):
     return x if f2sqr(x) == a else None
 
 
-n_in = n_out = 0
-for k in (1, 2, 3, 12345, R - 1, 0x1234567890abcdef1234567890abcdef):
-    T = G2.mul(O.G2_GEN, k)
-    assert fast_test(T) and old_test(T)
-    n_in += 1
-S = G2.mul(O.G2_GEN, 777)
-for t in range(1, 400):
-    xx = (t, 1)
-    y = f2sqrt(f2add(f2mul(f2sqr(xx), xx), B_TWIST))
-    if y is None:
-        continue
-    T = (xx, y)
-    for U in (T, G2.add(T, S), G2.mul(T, R), G2.mul(T, 10069)):      # raw, shifted by a subgroup point, pure cofactor part, a multiple
-        if U is None:
+def main():
+    n_in = n_out = 0
+    for k in (1, 2, 3, 12345, R - 1, 0x1234567890abcdef1234567890abcdef):
+        T = G2.mul(O.G2_GEN, k)
+        assert fast_test(T) and old_test(T)
+        n_in += 1
+    S = G2.mul(O.G2_GEN, 777)
+    for t in range(1, 400):
+        xx = (t, 1)
+        y = f2sqrt(f2add(f2mul(f2sqr(xx), xx), B_TWIST))
+        if y is None:
             continue
-        truth = G2.mul(U, R) is None
-        assert fast_test(U) == truth and old_test(U) == truth, (t, truth)
-        n_in += truth
-        n_out += (not truth)
-    if n_out >= 60:
-        break
-print("fast G2 membership test agrees with [r]T == O on", n_in, "subgroup points and", n_out, "points outside it")
+        T = (xx, y)
+        for U in (T, G2.add(T, S), G2.mul(T, R), G2.mul(T, 10069)):      # raw, shifted by a subgroup point, pure cofactor part, a multiple
+            if U is None:
+                continue
+            truth = G2.mul(U, R) is None
+            assert fast_test(U) == truth and old_test(U) == truth, (t, truth)
+            n_in += truth
+            n_out += (not truth)
+        if n_out >= 60:
+            break
+    print("fast G2 membership test agrees with [r]T == O on", n_in, "subgroup points and", n_out, "points outside it")
+
+
+if __name__ == "__main__":
+    main()
