@@ -277,6 +277,37 @@ int lzkp_verify_batch_device(lzkp_vk *vk, size_t n, const void *d_proofs, const 
  * the cooperative check available (1/0) */
 int lzkp_vk_info(const lzkp_vk *vk, uint64_t info[4]);
 
+/* ark-serialize's compressed form (Compress::Yes) next to the uncompressed one.  A compressed G1 point is x (32 B), a
+ * compressed G2 point x.c0 || x.c1 (64 B), flags in the top two bits of the last byte: 0x40 = infinity, 0x80 = y is the
+ * larger of y and -y (canonical integers; in Fq2 c1 first, then c0), both = invalid.  Objects keep the uncompressed
+ * field order and u64 length prefixes: Proof = A(32) || B(64) || C(32) = 128 B; VerifyingKey = 232 + 32 (n_pub + 1) B.
+ * Decoding takes one square root per point (Fq or Fq2), on the primary device, and checks no subgroup membership (ark's
+ * deserialize_compressed_unchecked): the loaders with validation and every verifier form check the decoded points as they
+ * check uncompressed ones, so decompress-then-load/verify decides what ark's validating compressed deserialization does.
+ * Compressing recomputes each sign from y (the input's 0x80 bit is not read); it is format work and checks no curve.
+ *
+ * lzkp_pk_load_compressed / lzkp_vk_load_compressed decode the key on the device in chunks (bounded scratch, released
+ * before the load) and pass the uncompressed bytes to lzkp_pk_load_ex / lzkp_vk_load: same options, validation, modes and
+ * multi-GPU replicas.  LZKP_E_INVALID for a key that does not parse or has a point that does not decode.
+ * lzkp_pk_compress / lzkp_vk_compress: uncompressed key bytes -> compressed; out == NULL sets *out_len only (from the
+ * layout, without reading the points).  Host byte work, no device. */
+int lzkp_pk_load_compressed(const uint8_t *pk_bytes, size_t len, int validate, const lzkp_pk_options *opt, lzkp_pk **out);
+int lzkp_vk_load_compressed(const uint8_t *vk_bytes, size_t len, lzkp_vk **out);
+int lzkp_pk_compress(const uint8_t *pk_bytes, size_t len, uint8_t *out, size_t cap, size_t *out_len);
+int lzkp_vk_compress(const uint8_t *vk_bytes, size_t len, uint8_t *out, size_t cap, size_t *out_len);
+/* Proofs n x 256 B <-> n x 128 B, ok_out[i] = 1 / 0.  Compressing: a row with a non-canonical coordinate or bad flags gets
+ * ok 0 and 128 B of 0xFF (host, no device).  Decompressing (primary device): a row that does not decode (non-canonical x,
+ * flags on x.c0, both flags, no point with that x) gets ok 0 and output bytes that every verifier form rejects as
+ * malformed (0xFF over the failing point).  The *_device forms take device buffers of the primary device (any alignment)
+ * and follow the contract of the other *_device entry points: enqueue-only on `stream`, LZKP_E_INVALID for a NULL buffer
+ * or a buffer that is not device memory of that device when n > 0, nothing enqueued for n == 0.  They draw no randomness,
+ * so a captured stream is accepted: lzkp_proofs_decompress_device then lzkp_verify_batch_device on one stream verifies
+ * compressed proofs with nothing copied through the host. */
+int lzkp_proofs_compress(size_t n, const uint8_t *proofs, uint8_t *out, uint8_t *ok_out);
+int lzkp_proofs_decompress(size_t n, const uint8_t *in, uint8_t *proofs_out, uint8_t *ok_out);
+int lzkp_proofs_compress_device(size_t n, const void *d_in, void *d_out, void *d_ok, void *stream);
+int lzkp_proofs_decompress_device(size_t n, const void *d_in, void *d_proofs_out, void *d_ok, void *stream);
+
 /* MiMC-5 commitment of a u64 (commit_value_snark), 32 B canonical LE.  Host arithmetic, no device. */
 int lzkp_commit_value_snark(uint64_t value, uint8_t out[32]);
 

@@ -59,6 +59,18 @@ extern "C" {
                              ok_out: *mut u8) -> c_int;
     pub fn lzkp_verify_batch_device(vk: *mut lzkp_vk, n: usize, d_proofs: *const c_void, d_public_inputs: *const c_void,
                                     n_pub: usize, d_ok: *mut c_void, stream: *mut c_void) -> c_int;
+    // ark-serialize compressed form (Compress::Yes): keys and proofs
+    pub fn lzkp_pk_load_compressed(pk: *const u8, len: usize, validate: c_int, opt: *const lzkp_pk_options,
+                                   out: *mut *mut lzkp_pk) -> c_int;
+    pub fn lzkp_vk_load_compressed(vk: *const u8, len: usize, out: *mut *mut lzkp_vk) -> c_int;
+    pub fn lzkp_pk_compress(pk: *const u8, len: usize, out: *mut u8, cap: usize, out_len: *mut usize) -> c_int;
+    pub fn lzkp_vk_compress(vk: *const u8, len: usize, out: *mut u8, cap: usize, out_len: *mut usize) -> c_int;
+    pub fn lzkp_proofs_compress(n: usize, proofs: *const u8, out: *mut u8, ok_out: *mut u8) -> c_int;
+    pub fn lzkp_proofs_decompress(n: usize, input: *const u8, proofs_out: *mut u8, ok_out: *mut u8) -> c_int;
+    pub fn lzkp_proofs_compress_device(n: usize, d_in: *const c_void, d_out: *mut c_void, d_ok: *mut c_void,
+                                       stream: *mut c_void) -> c_int;
+    pub fn lzkp_proofs_decompress_device(n: usize, d_in: *const c_void, d_proofs_out: *mut c_void, d_ok: *mut c_void,
+                                         stream: *mut c_void) -> c_int;
     pub fn lzkp_commit_value_snark(value: u64, out: *mut u8) -> c_int;
     pub fn lzkp_msm_g1(bases: *const u8, scalars: *const u8, n: usize, out: *mut u8) -> c_int;
     pub fn lzkp_msm_g2(bases: *const u8, scalars: *const u8, n: usize, out: *mut u8) -> c_int;

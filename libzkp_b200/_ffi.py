@@ -79,6 +79,14 @@ SIGNATURES = {
     "lzkp_vk_info": (_int, [_vp, C.POINTER(_u64)]),
     "lzkp_verify_batch": (_int, [_vp, _sz, _vp, _vp, _sz, _vp]),
     "lzkp_verify_batch_device": (_int, [_vp, _sz, _vp, _vp, _sz, _vp, _vp]),
+    "lzkp_pk_load_compressed": (_int, [_vp, _sz, _int, C.POINTER(PkOptions), C.POINTER(_vp)]),
+    "lzkp_vk_load_compressed": (_int, [_vp, _sz, C.POINTER(_vp)]),
+    "lzkp_pk_compress": (_int, [_vp, _sz, _vp, _sz, C.POINTER(_sz)]),
+    "lzkp_vk_compress": (_int, [_vp, _sz, _vp, _sz, C.POINTER(_sz)]),
+    "lzkp_proofs_compress": (_int, [_sz, _vp, _vp, _vp]),
+    "lzkp_proofs_decompress": (_int, [_sz, _vp, _vp, _vp]),
+    "lzkp_proofs_compress_device": (_int, [_sz, _vp, _vp, _vp, _vp]),
+    "lzkp_proofs_decompress_device": (_int, [_sz, _vp, _vp, _vp, _vp]),
     "lzkp_commit_value_snark": (_int, [_u64, _vp]),
 }
 

@@ -130,11 +130,15 @@ class ProvingKey:
     (src/backend/snark.rs:295-339), plus the circuit's R1CS matrices and NTT tables."""
 
     def __init__(self, pk_bytes: bytes, validate: bool = False, window_bits: int = 0,
-                 table_budget_bytes: int = 0, max_chunk: int = 0, shard_index: int = 0, shard_count: int = 0):
+                 table_budget_bytes: int = 0, max_chunk: int = 0, shard_index: int = 0, shard_count: int = 0,
+                 compressed: bool = False):
+        """compressed=True: pk_bytes is ark-serialize's compressed ProvingKey, decoded on the device
+        (lzkp_pk_load_compressed) and then loaded exactly as its uncompressed bytes would be."""
         self._h = C.c_void_p()
         buf = np.frombuffer(pk_bytes, dtype=np.uint8)
         opt = _ffi.PkOptions(window_bits, table_budget_bytes, max_chunk, shard_index, shard_count)
-        check(lib().lzkp_pk_load_ex(_p(buf), len(pk_bytes), int(validate), C.byref(opt), C.byref(self._h)))
+        load = lib().lzkp_pk_load_compressed if compressed else lib().lzkp_pk_load_ex
+        check(load(_p(buf), len(pk_bytes), int(validate), C.byref(opt), C.byref(self._h)))
         info = (C.c_uint64 * 8)()
         check(lib().lzkp_pk_info(self._h, info))
         (self.n_vars, self.n_inst, self.n_wit, self.n, self.window_bits, self.windows, self.table_bytes,
@@ -367,11 +371,13 @@ def generator_mul(group: int, scalars) -> np.ndarray:
 class VerifyingKey:
     """A verifying key resident on the device with e(alpha, beta) precomputed (lzkp_vk)."""
 
-    def __init__(self, vk_bytes: bytes):
+    def __init__(self, vk_bytes: bytes, compressed: bool = False):
+        """compressed=True: vk_bytes is ark-serialize's compressed VerifyingKey (lzkp_vk_load_compressed)."""
         self._h = C.c_void_p()
         buf = np.frombuffer(vk_bytes, dtype=np.uint8)
-        check(lib().lzkp_vk_load(_p(buf), len(vk_bytes), C.byref(self._h)))
-        self.n_pub = (len(vk_bytes) - 456) // 64 - 1
+        load = lib().lzkp_vk_load_compressed if compressed else lib().lzkp_vk_load
+        check(load(_p(buf), len(vk_bytes), C.byref(self._h)))
+        self.n_pub = self.info()[0]
 
     def verify_batch(self, proofs, public_inputs) -> np.ndarray:
         """proofs (n, 256) bytes; public_inputs (n, n_pub, 32) canonical bytes -> bool array."""
@@ -404,3 +410,52 @@ class VerifyingKey:
             self.close()
         except Exception:
             pass
+
+
+# ---- ark-serialize compressed form (Compress::Yes): proofs 128 B, G1 points 32 B, G2 points 64 B
+def _compress_key(fn, key_bytes: bytes) -> bytes:
+    buf = np.frombuffer(key_bytes, dtype=np.uint8)
+    n = C.c_size_t()
+    check(fn(_p(buf), len(key_bytes), None, 0, C.byref(n)))
+    out = np.zeros(n.value, np.uint8)
+    check(fn(_p(buf), len(key_bytes), _p(out), out.size, C.byref(n)))
+    return out.tobytes()
+
+
+def pk_compress(pk_bytes: bytes) -> bytes:
+    """Uncompressed ProvingKey bytes -> ark-serialize compressed bytes (lzkp_pk_compress, host byte work)."""
+    return _compress_key(lib().lzkp_pk_compress, pk_bytes)
+
+
+def vk_compress(vk_bytes: bytes) -> bytes:
+    """Uncompressed VerifyingKey bytes -> compressed bytes (lzkp_vk_compress, host byte work)."""
+    return _compress_key(lib().lzkp_vk_compress, vk_bytes)
+
+
+def proofs_compress(proofs) -> Tuple[np.ndarray, np.ndarray]:
+    """(n, 256) proofs -> ((n, 128) compressed proofs, ok bool[n]); ok False for a malformed row (host byte work)."""
+    proofs = _u8(proofs, 256)
+    n = proofs.shape[0]
+    out, ok = np.zeros((n, 128), np.uint8), np.zeros(n, np.uint8)
+    check(lib().lzkp_proofs_compress(n, _p(proofs), _p(out), _p(ok)))
+    return out, ok.astype(bool)
+
+
+def proofs_decompress(compressed) -> Tuple[np.ndarray, np.ndarray]:
+    """(n, 128) compressed proofs -> ((n, 256) proofs, ok bool[n]), decoded on the device; a row that does not decode
+    gets ok False and bytes every verifier form rejects."""
+    compressed = _u8(compressed, 128)
+    n = compressed.shape[0]
+    out, ok = np.zeros((n, 256), np.uint8), np.zeros(n, np.uint8)
+    check(lib().lzkp_proofs_decompress(n, _p(compressed), _p(out), _p(ok)))
+    return out, ok.astype(bool)
+
+
+def proofs_compress_device(n: int, d_proofs: int, d_out: int, d_ok: int, stream: int = 0) -> None:
+    """lzkp_proofs_compress_device: n x 256 B -> n x 128 B and n ok bytes, device pointers (ints), asynchronous."""
+    check(lib().lzkp_proofs_compress_device(n, d_proofs, d_out, d_ok, stream))
+
+
+def proofs_decompress_device(n: int, d_in: int, d_proofs: int, d_ok: int, stream: int = 0) -> None:
+    """lzkp_proofs_decompress_device: n x 128 B -> n x 256 B and n ok bytes, device pointers (ints), asynchronous."""
+    check(lib().lzkp_proofs_decompress_device(n, d_in, d_proofs, d_ok, stream))
