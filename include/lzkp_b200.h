@@ -308,6 +308,28 @@ int lzkp_proofs_decompress(size_t n, const uint8_t *in, uint8_t *proofs_out, uin
 int lzkp_proofs_compress_device(size_t n, const void *d_in, void *d_out, void *d_ok, void *stream);
 int lzkp_proofs_decompress_device(size_t n, const void *d_in, void *d_proofs_out, void *d_ok, void *stream);
 
+/* Groth16::<Bn254>::rerandomize_proof [ark-groth16, un-vendored], batched.  proofs / proofs_out n x 256 B,
+ * r1 / r2 n x 32 B canonical non-zero, ok_out[i] = 1 / 0.  proofs_out may equal proofs (in place).
+ * Per row, with the key's delta:  A' = r1^-1 A,  B' = r1 B + (r1 r2) delta,  C' = C + r2 A  - a fresh proof of the same
+ * statement, statistically indistinguishable from a newly generated one (BKSV20, ePrint 2020/811, Thm. 3); the result is
+ * written ark-serialize uncompressed (infinity flag when a point is the identity).  Like ark, the caller supplies the
+ * randomness: draw r1, r2 uniformly from the non-zero residues mod r for unlinkable presentations.
+ * A row gets ok 0 and 256 B of 0xFF (rejected as malformed by every verifier form), other rows unaffected, when
+ *   - a coordinate is >= q, x carries a flag, or y carries both flags;
+ *   - A, B or C is off its curve (the point at infinity is accepted);
+ *   - B is outside the r-torsion subgroup;
+ *   - r1 or r2 is 0 or >= r.
+ * These are the checks of Proof::deserialize_uncompressed (validating).  The host form stages rows through device memory
+ * in bounded chunks and blocks.  The *_device form takes device buffers of the key's device, proofs, factors and output
+ * 16-byte aligned, and follows the contract of lzkp_verify_batch_device (enqueue-only on `stream`; LZKP_E_INVALID for a
+ * NULL buffer, misalignment, host memory or another device's memory when n > 0; nothing enqueued for n == 0).  It only
+ * reads the key's delta and draws no randomness: calls on one key from several streams need no ordering, and a captured
+ * stream is accepted. */
+int lzkp_proofs_rerandomize(lzkp_vk *vk, size_t n, const uint8_t *proofs, const uint8_t *r1, const uint8_t *r2,
+                            uint8_t *proofs_out, uint8_t *ok_out);
+int lzkp_proofs_rerandomize_device(lzkp_vk *vk, size_t n, const void *d_proofs, const void *d_r1, const void *d_r2,
+                                   void *d_proofs_out, void *d_ok, void *stream);
+
 /* MiMC-5 commitment of a u64 (commit_value_snark), 32 B canonical LE.  Host arithmetic, no device. */
 int lzkp_commit_value_snark(uint64_t value, uint8_t out[32]);
 

@@ -71,6 +71,11 @@ extern "C" {
                                        stream: *mut c_void) -> c_int;
     pub fn lzkp_proofs_decompress_device(n: usize, d_in: *const c_void, d_proofs_out: *mut c_void, d_ok: *mut c_void,
                                          stream: *mut c_void) -> c_int;
+    pub fn lzkp_proofs_rerandomize(vk: *mut lzkp_vk, n: usize, proofs: *const u8, r1: *const u8, r2: *const u8,
+                                   proofs_out: *mut u8, ok_out: *mut u8) -> c_int;
+    pub fn lzkp_proofs_rerandomize_device(vk: *mut lzkp_vk, n: usize, d_proofs: *const c_void, d_r1: *const c_void,
+                                          d_r2: *const c_void, d_proofs_out: *mut c_void, d_ok: *mut c_void,
+                                          stream: *mut c_void) -> c_int;
     pub fn lzkp_commit_value_snark(value: u64, out: *mut u8) -> c_int;
     pub fn lzkp_msm_g1(bases: *const u8, scalars: *const u8, n: usize, out: *mut u8) -> c_int;
     pub fn lzkp_msm_g2(bases: *const u8, scalars: *const u8, n: usize, out: *mut u8) -> c_int;

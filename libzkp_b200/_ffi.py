@@ -87,6 +87,8 @@ SIGNATURES = {
     "lzkp_proofs_decompress": (_int, [_sz, _vp, _vp, _vp]),
     "lzkp_proofs_compress_device": (_int, [_sz, _vp, _vp, _vp, _vp]),
     "lzkp_proofs_decompress_device": (_int, [_sz, _vp, _vp, _vp, _vp]),
+    "lzkp_proofs_rerandomize": (_int, [_vp, _sz, _vp, _vp, _vp, _vp, _vp]),
+    "lzkp_proofs_rerandomize_device": (_int, [_vp, _sz, _vp, _vp, _vp, _vp, _vp, _vp]),
     "lzkp_commit_value_snark": (_int, [_u64, _vp]),
 }
 

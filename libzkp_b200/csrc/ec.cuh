@@ -245,6 +245,31 @@ LZ_HD GlvSplit glv_split(const Fr &k) {
     for (int i = 0; i < 4; i++) { o.k1[i] = k1[i]; o.k2[i] = k2[i]; }
     return o;
 }
+// ---- psi split of a BN254 scalar for G2: psi (pairing.cuh g2_psi) acts on the r-torsion of the twist as [lambda_psi],
+// lambda_psi = 6 x^2 = 0x6f4d8248eeb859fbf83e9682e87cfd46 (127 bits, below r).  For a canonical k < r:
+// k = k0 + k1 lambda_psi exactly, k0 = k mod lambda_psi, k1 = floor(k / lambda_psi), both below 2^127.  The quotient
+// estimate floor(k M / 2^256) with M = floor(2^256 / lambda_psi) is the quotient or one less; one conditional
+// subtraction settles it.
+LZ_HD void psi_split(const uint32_t (&k)[8], uint32_t (&k0)[4], uint32_t (&k1)[4]) {
+    const uint32_t L[8] = {0xe87cfd46u, 0xf83e9682u, 0xeeb859fbu, 0x6f4d8248u, 0u, 0u, 0u, 0u};
+    const uint32_t L4[4] = {0xe87cfd46u, 0xf83e9682u, 0xeeb859fbu, 0x6f4d8248u};
+    const uint32_t M[5] = {0xc8e01941u, 0x2cb62031u, 0xa773d2d5u, 0x4ccef014u, 0x00000002u};
+    uint32_t t[13], q[4], ql[8], rem[8], d[8];
+    mul_limbs<13, 8, 5>(t, k, M);
+#pragma unroll
+    for (int i = 0; i < 4; i++) q[i] = t[8 + i];          // t[12] == 0 for k < r
+    mul_limbs<8, 4, 4>(ql, q, L4);
+    sub8(rem, k, ql);                                     // k - q lambda_psi < 2 lambda_psi
+    const bool over = sub8(d, rem, L) == 0;               // rem >= lambda_psi
+    uint32_t c = over ? 1u : 0u;
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        k0[i] = over ? d[i] : rem[i];
+        const uint64_t s = (uint64_t)q[i] + c;
+        k1[i] = (uint32_t)s;
+        c = (uint32_t)(s >> 32);
+    }
+}
 // k * p for a 128-bit magnitude
 template <class F>
 LZ_COLD XYZZ<F> scalar_mul_u128(const XYZZ<F> &p, const uint32_t (&k)[4]) {
@@ -297,6 +322,57 @@ static LZ_COLD XYZZ<Fq> scalar_mul_glv64(const XYZZ<Fq> &p, const uint32_t (&k)[
                 XYZZ<Fq> q = T[(d < 0 ? -d : d) - 1];
                 if (h) q.x = q.x * beta;
                 if (d < 0) q.y = q.y.neg();
+                acc.add_cold(q);
+            }
+        }
+    }
+    return acc;
+}
+// T[i] = (i + 1) p, i < 8: the table of a signed 4-bit window ladder
+template <class F>
+LZ_COLD void window_table(XYZZ<F> (&T)[8], const XYZZ<F> &p) {
+    T[0] = p;
+    T[1] = p;
+    T[1].dbl_cold();
+#pragma unroll 1
+    for (int i = 2; i < 8; i++) {
+        T[i] = T[i - 1];
+        T[i].add_cold(p);
+    }
+}
+// sum_j (+-k_j) P_j over N bases with 128-bit magnitudes k_j: ONE signed 4-bit window ladder (33 windows: 132 doublings
+// shared by all bases, at most one addition per base and window).  T[j] = window_table(P_j); bit j of `neg` negates P_j.
+// With P_j = P and an endomorphism image of P (phi on G1, psi on G2) this is a GLV / psi-split scalar multiplication.
+template <class F, int N>
+LZ_COLD XYZZ<F> joint_mul_u128(const XYZZ<F> (&T)[N][8], const uint32_t (&k)[N][4], uint32_t neg) {
+    uint32_t carries[N], top = 0;
+#pragma unroll 1
+    for (int j = 0; j < N; j++) {
+        uint32_t c = 0, m = 0;
+#pragma unroll 1
+        for (int i = 0; i < 32; i++) {
+            const uint32_t v = ((k[j][i >> 3] >> ((i & 7) * 4)) & 15u) + c;
+            c = v >= 8u ? 1u : 0u;
+            m |= c << i;
+        }
+        carries[j] = m;
+        top |= c << j;
+    }
+    XYZZ<F> acc = XYZZ<F>::inf();
+#pragma unroll 1
+    for (int i = 32; i >= 0; i--) {
+        acc.dbl_cold(); acc.dbl_cold(); acc.dbl_cold(); acc.dbl_cold();
+#pragma unroll 1
+        for (int j = 0; j < N; j++) {
+            int d;
+            if (i == 32) d = (int)((top >> j) & 1u);
+            else {
+                const uint32_t cin = i ? (carries[j] >> (i - 1)) & 1u : 0u, cout = (carries[j] >> i) & 1u;
+                d = (int)(((k[j][i >> 3] >> ((i & 7) * 4)) & 15u) + cin) - (int)(16u * cout);
+            }
+            if (d != 0) {
+                XYZZ<F> q = T[j][(d < 0 ? -d : d) - 1];
+                if ((d < 0) != (((neg >> j) & 1u) != 0)) q.y = q.y.neg();
                 acc.add_cold(q);
             }
         }

@@ -1778,6 +1778,19 @@ int lzkp_verify_batch_device(lzkp_vk *vk, size_t n, const void *d_proofs, const 
     return verify_batch_device(vk->v, n, (const uint8_t *)d_proofs, (const uint8_t *)d_public_inputs, n_pub, (uint8_t *)d_ok,
                                (cudaStream_t)stream);
 }
+int lzkp_proofs_rerandomize(lzkp_vk *vk, size_t n, const uint8_t *proofs, const uint8_t *r1, const uint8_t *r2,
+                            uint8_t *proofs_out, uint8_t *ok_out) {
+    if (!vk || (n && (!proofs || !r1 || !r2 || !proofs_out || !ok_out))) return fail(LZKP_E_INVALID, "null argument");
+    TRY(ensure_device());
+    return proofs_rerandomize(vk->v, n, proofs, r1, r2, proofs_out, ok_out);
+}
+int lzkp_proofs_rerandomize_device(lzkp_vk *vk, size_t n, const void *d_proofs, const void *d_r1, const void *d_r2,
+                                   void *d_proofs_out, void *d_ok, void *stream) {
+    if (!vk || (n && (!d_proofs || !d_r1 || !d_r2 || !d_proofs_out || !d_ok))) return fail(LZKP_E_INVALID, "null argument");
+    TRY(ensure_device());
+    return proofs_rerandomize_device(vk->v, n, (const uint8_t *)d_proofs, (const uint8_t *)d_r1, (const uint8_t *)d_r2,
+                                     (uint8_t *)d_proofs_out, (uint8_t *)d_ok, (cudaStream_t)stream);
+}
 
 int lzkp_commit_value_snark(uint64_t value, uint8_t out[32]) {
     if (!out) return fail(LZKP_E_INVALID, "null argument");

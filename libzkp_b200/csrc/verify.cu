@@ -15,6 +15,7 @@
 // and the combined form's scalar sums from k_rlc_input_sums.
 // lzkp_verify_batch_device runs the same stages on the caller's stream from device buffers; its coefficients come from
 // k_rlc_rho and its failing groups are listed by k_rlc_failed and re-verified by the Listed instantiations of the forms.
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -25,6 +26,7 @@
 #include "host_util.h"
 #include "coop.cuh"
 #include "pairing.cuh"
+#include "proof_read.cuh"
 #include "verify.h"
 
 namespace lzkp {
@@ -36,43 +38,6 @@ struct VkDev {
     G2Affine beta, gamma_neg, delta_neg;
     Fq12 alpha_beta;                 // e(alpha, beta), filled by k_vk_prepare
 };
-
-__device__ __forceinline__ bool read_fq_canonical(const uint8_t *b, Fq &out, uint32_t &flags) {
-    const uint4 *s = reinterpret_cast<const uint4 *>(b);
-    uint4 lo = s[0], hi = s[1];
-    flags = hi.w >> 30;
-    hi.w &= 0x3FFFFFFFu;
-    Fq c;
-    c.l[0] = lo.x; c.l[1] = lo.y; c.l[2] = lo.z; c.l[3] = lo.w; c.l[4] = hi.x; c.l[5] = hi.y; c.l[6] = hi.z; c.l[7] = hi.w;
-    uint32_t d[8];
-    Fq m = Fq::modulus();
-    bool ok = sub8(d, c.l, m.l) != 0;          // c < q
-    out = Fq::from_canonical(c);
-    return ok;
-}
-// ark-serialize uncompressed, validating: canonical coordinates, on the curve (infinity flag accepted)
-__device__ __noinline__ bool read_g1_checked(const uint8_t *b, G1Affine &p) {
-    uint32_t f0, f1;
-    bool ok = read_fq_canonical(b, p.x, f0) & read_fq_canonical(b + 32, p.y, f1);
-    if (f0) ok = false;
-    if (f1 & 1u) { p = G1Affine::inf(); return ok; }        // infinity flag (bit 6 of the last byte)
-    return ok && g1_on_curve(p);
-}
-__device__ __noinline__ bool read_g2_on_curve(const uint8_t *b, G2Affine &p) {
-    uint32_t f0, f1, f2, f3;
-    bool ok = read_fq_canonical(b, p.x.c0, f0) & read_fq_canonical(b + 32, p.x.c1, f1) &
-              read_fq_canonical(b + 64, p.y.c0, f2) & read_fq_canonical(b + 96, p.y.c1, f3);
-    if (f0 | f1 | f2) ok = false;
-    if (f3 & 1u) { p = G2Affine::inf(); return ok; }
-    return ok && g2_on_curve(p);
-}
-__device__ __noinline__ bool read_g2_checked(const uint8_t *b, G2Affine &p) {
-    if (!read_g2_on_curve(b, p)) return false;
-    if (p.is_inf()) return true;
-    // subgroup check (deserialize_uncompressed validates it): pairing.cuh g2_subgroup_from_xp, one 63-bit ladder
-    const uint32_t x[2] = {kBnXLimbs[0], kBnXLimbs[1]};
-    return g2_subgroup_from_xp(p, scalar_mul_window<Fq2, 2>(G2XYZZ::from_affine(p), x));
-}
 
 // e(alpha, beta) once per key (what process_vk precomputes)
 // What VerifyingKey::deserialize_uncompressed (Validate::Yes, snark.rs:66) checks: every point of the key is on its
@@ -1161,6 +1126,9 @@ int vk_load(const uint8_t *bytes, size_t len, VerifyingKeyDev **out) {
     return LZKP_OK;
 }
 void vk_free(VerifyingKeyDev *V) { delete V; }
+const G2Affine *vk_delta_neg(const VerifyingKeyDev *V) {
+    return reinterpret_cast<const G2Affine *>(V->vk.as<char>() + offsetof(VkDev, delta_neg));
+}
 uint32_t vk_num_inputs(const VerifyingKeyDev *V) { return V->n_pub; }
 void vk_info(const VerifyingKeyDev *V, uint64_t info[4]) {
     info[0] = V->n_pub;
@@ -1365,7 +1333,7 @@ int verify_batch(VerifyingKeyDev *V, size_t n, const uint8_t *proofs, const uint
 }
 
 // Device memory of the key's device, not host memory (cudaPointerGetAttributes: unregistered or pinned host memory).
-static int check_device_buffer(const VerifyingKeyDev *V, const void *p, const char *what) {
+int check_device_buffer(const VerifyingKeyDev *V, const void *p, const char *what) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
         cudaGetLastError();

@@ -394,6 +394,39 @@ class VerifyingKey:
         pointers (ints) on the key's device; asynchronous on `stream`.  Refused on a stream that is being captured."""
         check(lib().lzkp_verify_batch_device(self._h, n, d_proofs, d_inputs, n_pub, d_ok, stream))
 
+    def rerandomize(self, proofs, r1=None, r2=None) -> Tuple[np.ndarray, np.ndarray]:
+        """ark-groth16's rerandomize_proof on n proofs: (n, 256) proofs -> ((n, 256) fresh proofs of the same statements,
+        ok bool[n]).  r1, r2 are (n, 32) canonical non-zero factors; a missing one is drawn from the OS CSPRNG
+        (snark.OsRng, zeros redrawn as ark's loop does).  A malformed row, or one with a factor 0 or >= r, gets ok False
+        and bytes every verifier form rejects."""
+        from .snark import OsRng
+        proofs = _u8(proofs, 256)
+        n = proofs.shape[0]
+
+        def factors(f):
+            if f is not None:
+                f = _u8(f, 32)
+                if f.shape[0] != n:
+                    raise ValueError("r1, r2 must hold one factor per proof")
+                return f
+            f = OsRng().scalars(n)
+            while True:
+                zero = ~f.any(axis=1)
+                if not zero.any():
+                    return f
+                f[zero] = OsRng().scalars(int(zero.sum()))
+
+        r1, r2 = factors(r1), factors(r2)
+        out, ok = np.zeros((n, 256), np.uint8), np.zeros(n, np.uint8)
+        check(lib().lzkp_proofs_rerandomize(self._h, n, _p(proofs), _p(r1), _p(r2), _p(out), _p(ok)))
+        return out, ok.astype(bool)
+
+    def rerandomize_device(self, n: int, d_proofs: int, d_r1: int, d_r2: int, d_out: int, d_ok: int,
+                           stream: int = 0) -> None:
+        """lzkp_proofs_rerandomize_device: proofs and output (n x 256 B, d_out may be d_proofs), factors (n x 32 B) and
+        ok (n bytes) are device pointers (ints) on the key's device, 16-byte aligned; asynchronous on `stream`."""
+        check(lib().lzkp_proofs_rerandomize_device(self._h, n, d_proofs, d_r1, d_r2, d_out, d_ok, stream))
+
     def info(self):
         """(n_pub, table bytes, latency form available, combined form available) of the loaded key."""
         v = (C.c_uint64 * 4)()
