@@ -61,31 +61,6 @@ __device__ __forceinline__ Affine<F> gather_point(const Affine<F> *table, uint32
     return pt;
 }
 
-// Signed c-bit window recoding by the offset trick: s' = s + K with K = sum_w 2^(c*w + c-1); the
-// unsigned windows u_w of s' give d_w = u_w - 2^(c-1) in [-2^(c-1), 2^(c-1)), independently per
-// window (no carry chain between windows).  Needs c * W >= 255 so that s' < 2^(c*W).
-__device__ __forceinline__ void recode_offset(const Fr &s, uint32_t c, uint32_t W, uint32_t (&v)[10]) {
-    uint64_t carry = 0;
-#pragma unroll
-    for (int i = 0; i < 9; i++) {
-        uint32_t kl = 0;                      // limb i of K
-        for (uint32_t w = 0; w < W; w++) {
-            uint32_t bit = c * w + c - 1;
-            if ((bit >> 5) == (uint32_t)i) kl |= 1u << (bit & 31);
-        }
-        uint64_t t = (uint64_t)(i < 8 ? s.l[i] : 0u) + kl + carry;
-        v[i] = (uint32_t)t;
-        carry = t >> 32;
-    }
-    v[9] = 0;
-}
-__device__ __forceinline__ int recoded_digit(const uint32_t (&v)[10], uint32_t c, uint32_t w) {
-    uint32_t bit = c * w, li = bit >> 5, sh = bit & 31;
-    uint64_t two = ((uint64_t)v[li + 1] << 32) | v[li];
-    uint32_t u = (uint32_t)(two >> sh) & ((1u << c) - 1u);
-    return (int)u - (int)(1u << (c - 1));
-}
-
 // ---------------------------------------------------------------- ark-serialize writers
 __device__ __forceinline__ void put_fq(uint8_t *out, const Fq &canon, uint32_t flags) {
     uint4 *o = reinterpret_cast<uint4 *>(out);

@@ -184,7 +184,8 @@ LZ_COLD XYZZ<F> scalar_mul(const XYZZ<F> &p, const Fr &k_canonical) {
 // eigenvalue of the G1 endomorphism phi(x, y) = (beta * x, y).  Halves the serial doubling chain of a
 // variable-base scalar multiplication (proof assembly: s * A and r * B1).  Lattice basis (a1, b1), (a2, b2)
 // from the extended Euclidean algorithm on (r, lambda); c_i = floor(k * g_i / 2^256) with g_i = floor(2^256 *
-// {b2, -b1} / r) (checked against exact rounding over 2 * 10^5 scalars: |k1|, |k2| <= 2^127).
+// {b2, -b1} / r) (checked against exact rounding over 2 * 10^5 scalars: |k1|, |k2| <= 2^127; at the lattice basis
+// and the rounding boundaries of c_i by tests/test_curve_prims_host.py).
 struct GlvSplit {
     uint32_t k1[4], k2[4];
     bool neg1, neg2, ok;      // ok == false: magnitudes did not fit 128 bits (never observed) -> caller uses the plain ladder
@@ -394,6 +395,31 @@ LZ_HD Fr glv64_coefficient(const uint32_t (&k)[4]) {
     k1.l[0] = k[0]; k1.l[1] = k[1];
     k2.l[0] = k[2]; k2.l[1] = k[3];
     return k1 + k2 * glv_lambda_mont();          // (k2)(lambda R) R^-1 = k2 lambda, canonical
+}
+
+// Signed c-bit window recoding by the offset trick: s' = s + K with K = sum_w 2^(c*w + c-1); the
+// unsigned windows u_w of s' give d_w = u_w - 2^(c-1) in [-2^(c-1), 2^(c-1)), independently per
+// window (no carry chain between windows).  Needs c * W >= 255 so that s' < 2^(c*W).
+LZ_HD void recode_offset(const Fr &s, uint32_t c, uint32_t W, uint32_t (&v)[10]) {
+    uint64_t carry = 0;
+#pragma unroll
+    for (int i = 0; i < 9; i++) {
+        uint32_t kl = 0;                      // limb i of K
+        for (uint32_t w = 0; w < W; w++) {
+            uint32_t bit = c * w + c - 1;
+            if ((bit >> 5) == (uint32_t)i) kl |= 1u << (bit & 31);
+        }
+        uint64_t t = (uint64_t)(i < 8 ? s.l[i] : 0u) + kl + carry;
+        v[i] = (uint32_t)t;
+        carry = t >> 32;
+    }
+    v[9] = 0;
+}
+LZ_HD int recoded_digit(const uint32_t (&v)[10], uint32_t c, uint32_t w) {
+    uint32_t bit = c * w, li = bit >> 5, sh = bit & 31;
+    uint64_t two = ((uint64_t)v[li + 1] << 32) | v[li];
+    uint32_t u = (uint32_t)(two >> sh) & ((1u << c) - 1u);
+    return (int)u - (int)(1u << (c - 1));
 }
 
 using G1Affine = Affine<Fq>;

@@ -263,7 +263,7 @@ static uint32_t fit_item_len(const std::vector<std::vector<BaseRef>> &msms, uint
     return best;
 }
 
-// Signed c-bit windows of an Fr scalar by the offset trick (dev_util.cuh recode_offset): s + K must stay below
+// Signed c-bit windows of an Fr scalar by the offset trick (ec.cuh recode_offset): s + K must stay below
 // 2^(c*W) with K = sum_w 2^(c*w + c-1) < 2^(c*W - 1) * (1 + 2^(1-c)).  BN254's r is 0.756 * 2^254, so c * W >= 255
 // is enough: W = ceil(255 / c) (15 windows at c = 17, 16 at c = 16, 17 at c = 15).
 static inline uint32_t window_count(int c) { return (uint32_t)((255 + c - 1) / c); }

@@ -84,7 +84,8 @@ __global__ void __launch_bounds__(256) k_msm_digits(const Fr *__restrict__ scala
 // windows - the window combination's chain of dependent doublings drops from c (W - 1) = 240 to 128 and the number of
 // bucket sets to reduce from 16 to 9 - for the same number of (point, window) pairs.
 // Magnitudes of the lattice split stay below ~2^128 (ec.cuh glv_split: never above 2^127 over 2 * 10^5 scalars);
-// the W = ceil(129 / c) + ... windows used here hold anything below 2^(c W - 1), and a split beyond that is counted in
+// the W = ceil(130 / c) windows used here hold anything below 2^(c W - 2) (s + K < 2^(c W) with the recoding offset
+// K < 2^(c W - 1) (1 + 2^(1-c)); c W >= 130, so every 128-bit magnitude fits), and a split beyond that is counted in
 // `bad` like a non-canonical scalar rather than silently mis-added.
 __device__ __forceinline__ void glv_split_wide(const Fr &k, Fr &m1, bool &neg1, Fr &m2, bool &neg2) {
     const uint32_t G1C[5] = {0x00ff6565u, 0x5398fd03u, 0xa773d2d2u, 0x4ccef014u, 0x00000002u};
@@ -130,7 +131,7 @@ __global__ void __launch_bounds__(256) k_msm_digits_glv(const Fr *__restrict__ s
     Fr m[2];
     bool neg[2];
     glv_split_wide(s, m[0], neg[0], m[1], neg[1]);
-    const uint32_t top = c * W - 1;                       // magnitudes must stay below 2^top for the offset recoding
+    const uint32_t top = c * W - 2;                       // magnitudes must stay below 2^top for the offset recoding
     for (int h = 0; h < 2; h++) {
         uint32_t over = 0;
         for (uint32_t b = top >> 5; b < 8; b++) over |= b == (top >> 5) ? (m[h].l[b] >> (top & 31)) : m[h].l[b];

@@ -18,6 +18,9 @@ __device__ void run_family(int code, const uint32_t *in, uint32_t *out) {
     else if (FAM == prim::FAM_FQ2) prim::fq2_op(code, in, out);
     else if (FAM == prim::FAM_TOWER) prim::tower_op(code, in, out);
     else if (FAM == prim::FAM_PAIRING) prim::pairing_op(code, in, out);
+    else if (FAM == prim::FAM_G1_CURVE) prim::curve_op<Fq>(code, in, out);
+    else if (FAM == prim::FAM_G2_CURVE) prim::curve_op<Fq2>(code, in, out);
+    else if (FAM == prim::FAM_SCALAR) prim::scalar_op(code, in, out);
     else prim::g2_op(code, in, out);
 }
 // one kernel per family, so that the field operations are not compiled beside the pairing
@@ -145,6 +148,9 @@ int prim_launch(int family, int code, const void *in, void *out, int n, cudaStre
         case prim::FAM_TOWER: return (int)launch_prim<prim::FAM_TOWER>(code, in, out, n, st);
         case prim::FAM_PAIRING: return (int)launch_prim<prim::FAM_PAIRING>(code, in, out, n, st);
         case prim::FAM_G2: return (int)launch_prim<prim::FAM_G2>(code, in, out, n, st);
+        case prim::FAM_G1_CURVE: return (int)launch_prim<prim::FAM_G1_CURVE>(code, in, out, n, st);
+        case prim::FAM_G2_CURVE: return (int)launch_prim<prim::FAM_G2_CURVE>(code, in, out, n, st);
+        case prim::FAM_SCALAR: return (int)launch_prim<prim::FAM_SCALAR>(code, in, out, n, st);
         default: return (int)cudaErrorInvalidValue;
     }
 }

@@ -9,14 +9,26 @@
 #include <stddef.h>
 
 #include "../../libzkp_b200/csrc/pairing.cuh"
+#ifdef __CUDACC__
+#include "../../libzkp_b200/csrc/dev_util.cuh"
+#endif
 
 namespace prim {
 using namespace lzkp;
 
-enum Family { FAM_FR = 0, FAM_FQ = 1, FAM_FQ2 = 2, FAM_TOWER = 3, FAM_PAIRING = 4, FAM_G2 = 5, FAM_COUNT = 6 };
+enum Family {
+    FAM_FR = 0, FAM_FQ = 1, FAM_FQ2 = 2, FAM_TOWER = 3, FAM_PAIRING = 4, FAM_G2 = 5,
+    FAM_G1_CURVE = 6, FAM_G2_CURVE = 7, FAM_SCALAR = 8, FAM_COUNT = 9
+};
 // words per input / output record of each family
-LZ_HD constexpr int in_words(int f) { return f == FAM_TOWER ? 192 : f == FAM_PAIRING ? 200 : 32; }
-LZ_HD constexpr int out_words(int f) { return f <= FAM_FQ ? 17 : f == FAM_FQ2 ? 16 : f == FAM_G2 ? 33 : 96; }
+LZ_HD constexpr int in_words(int f) {
+    return f == FAM_TOWER ? 192 : f == FAM_PAIRING ? 200 : f == FAM_G1_CURVE ? 96 : f == FAM_G2_CURVE ? 176
+         : f == FAM_SCALAR ? 16 : 32;
+}
+LZ_HD constexpr int out_words(int f) {
+    return f <= FAM_FQ ? 17 : f == FAM_FQ2 ? 16 : f == FAM_G2 ? 33 : f == FAM_G1_CURVE ? 65 : f == FAM_G2_CURVE ? 129
+         : f == FAM_SCALAR ? 32 : 96;
+}
 
 template <class T> LZ_HD T load(const uint32_t *p) {
     T v;
@@ -157,6 +169,119 @@ LZ_HD void g2_op(int, const uint32_t *in, uint32_t *out) {
     out[32] = g2_subgroup_from_xp(p, xp) ? 1u : 0u;
 }
 
+// ec.cuh's group law and ladders, F = Fq (FAM_G1_CURVE) or Fq2 (FAM_G2_CURVE).  With E = the words of one F (8 / 16):
+// in = acc (XYZZ, 4E) | P (affine, 2E) | Q (XYZZ, 4E) | s (8) | aux (8).  out = an XYZZ (4E; an affine result in the
+// first 2E) | a second XYZZ (4E) | a flag.  Coordinates are Montgomery limbs; the ladders read s as plain limbs.
+//   0 acc.madd(P)   1 acc.add(Q)   2 acc.add_cold(Q)   3 acc.dbl()   4 dbl_affine(P)   5 from_affine(P)   6 acc.to_affine()
+//   7 acc.neg()   8 G1: acc.madd_lazy(P), then canonical() (second XYZZ: the redundant form before it)
+//   9 on_curve(P) (flag)   10 scalar_mul_window<F, 8>(acc, s)   11 scalar_mul_window<F, 4>(acc, s[0..3])
+//   12 joint_mul_u128<F, 2>(T, {s[0..3], s[4..7]}, aux[0]) with T[0] = window_table(acc) and T[1] its image under phi
+//      (G1: x -> beta x, as rerandomize.cu's g1_rerandomize) or psi (G2: g2_psi, as g2_rerandomize)
+//   13 G1: scalar_mul_glv64(acc, s[0..3])
+//   14 gather_point(table, aux[1], aux[2], (int)aux[3]) on the record's first words read as an Affine<F> table.
+//      gather_point (dev_util.cuh) is device code: the host build runs a restatement of it here, so only the device
+//      build of this operation tests the library (against the restatement bit for bit, then the oracle).
+template <class F>
+LZ_HD void curve_op(int code, const uint32_t *in, uint32_t *out) {
+    constexpr int E = (int)(sizeof(F) / 4);
+    XYZZ<F> acc = load<XYZZ<F>>(in);
+    const Affine<F> P = load<Affine<F>>(in + 4 * E);
+    const XYZZ<F> Q = load<XYZZ<F>>(in + 6 * E);
+    const uint32_t *s = in + 10 * E, *aux = in + 10 * E + 8;
+    XYZZ<F> r = XYZZ<F>::inf(), r2 = XYZZ<F>::inf();
+    for (int i = 0; i < 8 * E + 1; i++) out[i] = 0;
+    uint32_t k8[8], k4[4], kk[2][4];
+    for (int i = 0; i < 8; i++) { k8[i] = s[i]; kk[i >> 2][i & 3] = s[i]; }
+    for (int i = 0; i < 4; i++) k4[i] = s[i];
+    bool affine_out = false;
+    Affine<F> a = Affine<F>::inf();
+    switch (code) {
+        case 0: r = acc; r.madd(P); break;
+        case 1: r = acc; r.add(Q); break;
+        case 2: r = acc; r.add_cold(Q); break;
+        case 3: r = acc; r.dbl(); break;
+        case 4: r = XYZZ<F>::dbl_affine(P); break;
+        case 5: r = XYZZ<F>::from_affine(P); break;
+        case 6: a = acc.to_affine(); affine_out = true; break;
+        case 7: r = acc.neg(); break;
+        case 8:
+            if constexpr (E == 8) { r2 = acc; r2.madd_lazy(P); r = r2.canonical(); }
+            break;
+        case 9:
+            if constexpr (E == 8) out[8 * E] = g1_on_curve(P) ? 1u : 0u;
+            else out[8 * E] = g2_on_curve(P) ? 1u : 0u;
+            return;
+        case 10: r = scalar_mul_window<F, 8>(acc, k8); break;
+        case 11: r = scalar_mul_window<F, 4>(acc, k4); break;
+        case 12: {
+            XYZZ<F> T[2][8];
+            window_table(T[0], acc);
+            for (int i = 0; i < 8; i++) {
+                if constexpr (E == 8) {
+                    Fq beta;
+                    for (int j = 0; j < 8; j++) beta.l[j] = FqParams::BETA(j);
+                    T[1][i] = T[0][i];
+                    T[1][i].x = T[1][i].x * beta;
+                } else {
+                    T[1][i] = g2_psi(T[0][i]);
+                }
+            }
+            r = joint_mul_u128<F, 2>(T, kk, aux[0]);
+            break;
+        }
+        case 13:
+            if constexpr (E == 8) r = scalar_mul_glv64(acc, k4);
+            break;
+        case 14: {
+            const int d = (int)aux[3];
+#ifdef __CUDA_ARCH__
+            a = gather_point(reinterpret_cast<const Affine<F> *>(in), aux[1], aux[2], d);
+#else
+            a = load<Affine<F>>(in + 2 * E * (aux[1] * aux[2] + (uint32_t)(d < 0 ? -d : d) - 1u));
+            if (d < 0) a.y = a.y.neg();
+#endif
+            affine_out = true;
+            break;
+        }
+        default: break;
+    }
+    if (affine_out) { store(out, a); return; }
+    store(out, r);
+    store(out + 4 * E, r2);
+}
+
+// Scalar splits and recodings of ec.cuh.  in = s (8 words, plain limbs) | c | W (6 words unused); out = 32 words.
+//   0 glv_split(s): k1 (4) | k2 (4) | neg1 | neg2 | ok   1 psi_split(s): k0 (4) | k1 (4)
+//   2 glv64_coefficient(s[0..3]) (canonical)   3 recode_offset(s, c, W), then recoded_digit(c, w) for w < W (int32)
+LZ_HD void scalar_op(int code, const uint32_t *in, uint32_t *out) {
+    Fr s;
+    uint32_t k8[8], k4[4], a[4], b[4];
+    for (int i = 0; i < 8; i++) { s.l[i] = in[i]; k8[i] = in[i]; }
+    for (int i = 0; i < 4; i++) k4[i] = in[i];
+    for (int i = 0; i < 32; i++) out[i] = 0;
+    switch (code) {
+        case 0: {
+            const GlvSplit g = glv_split(s);
+            for (int i = 0; i < 4; i++) { out[i] = g.k1[i]; out[4 + i] = g.k2[i]; }
+            out[8] = g.neg1; out[9] = g.neg2; out[10] = g.ok;
+            break;
+        }
+        case 1:
+            psi_split(k8, a, b);
+            for (int i = 0; i < 4; i++) { out[i] = a[i]; out[4 + i] = b[i]; }
+            break;
+        case 2: store(out, glv64_coefficient(k4)); break;
+        case 3: {
+            const uint32_t c = in[8], W = in[9] < 32 ? in[9] : 32;
+            uint32_t v[10];
+            recode_offset(s, c, W, v);
+            for (uint32_t w = 0; w < W; w++) out[w] = (uint32_t)recoded_digit(v, c, w);
+            break;
+        }
+        default: break;
+    }
+}
+
 LZ_HD void run(int family, int code, const uint32_t *in, uint32_t *out) {
     switch (family) {
         case FAM_FR: field_op<Fr>(code, in, out); break;
@@ -164,6 +289,9 @@ LZ_HD void run(int family, int code, const uint32_t *in, uint32_t *out) {
         case FAM_FQ2: fq2_op(code, in, out); break;
         case FAM_TOWER: tower_op(code, in, out); break;
         case FAM_PAIRING: pairing_op(code, in, out); break;
+        case FAM_G1_CURVE: curve_op<Fq>(code, in, out); break;
+        case FAM_G2_CURVE: curve_op<Fq2>(code, in, out); break;
+        case FAM_SCALAR: scalar_op(code, in, out); break;
         default: g2_op(code, in, out); break;
     }
 }

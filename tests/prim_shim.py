@@ -13,7 +13,7 @@ import numpy as np
 from conftest import ROOT
 
 R = 1 << 256
-FAM_FR, FAM_FQ, FAM_FQ2, FAM_TOWER, FAM_PAIRING, FAM_G2 = range(6)
+FAM_FR, FAM_FQ, FAM_FQ2, FAM_TOWER, FAM_PAIRING, FAM_G2, FAM_G1_CURVE, FAM_G2_CURVE, FAM_SCALAR = range(9)
 SHIM = os.path.join(ROOT, "tests", "device_shim")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-shared"]
 
@@ -41,7 +41,7 @@ _BUILT = {}
 
 
 def device(tmp_path_factory):
-    """the device shim, compiled once per session (it takes about two minutes)"""
+    """the device shim, compiled once per session (under a minute)"""
     if "device" not in _BUILT:
         _BUILT["device"] = Device(compile_device(tmp_path_factory.mktemp("prim_dev")))
     return _BUILT["device"]
